@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (ours; torchrun for N > 1)
     python bench.py --impl reference --gpus N --steps K ...  (CPU arm: the oracle port)
+    python bench.py ... --dump-outputs DIR                   (+ the state after the last timed step)
 
 A "step" is one verlet_step! (src/current/wcsph_perturbed_witch.jl:309-332) over the
 whole particle set.  Workload: BASELINE.json config 4, the 3D bell-hill mountain wave
@@ -24,6 +25,7 @@ import numpy as np
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True   # the benchmark leaves the tree as it found it (which may be read-only)
 
 # 3D: algorithmic bytes per particle of the unfused canonical kernels (SURVEY.md §8d)
 BYTES_3D = {"K_A": 117, "K_S": 183, "K_B": 72, "K_C": 113, "step": 485}
@@ -66,7 +68,13 @@ def parse():
                     help="SPHMW_FLAG_*: 0 strict arithmetic (default: FP64 sums bit-identical to the oracle), "
                          "1 FAST_MATH, 2 CELL_PAIRS, +4 NO_PAIR_LIST (walk the cells in every pass), +16 NO_PRETEST, "
                          "+64 TILES (shared-memory tiles, experimental), +128 NO_PACKED_RECORDS (SoA gathers)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the particle state after the last timed step to DIR/<field>.npy (float64, "
+                         "global index order; a fixed sample of large runs), to compare two builds")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def measured_peaks():
@@ -154,10 +162,11 @@ class ClockSampler:
 
 
 # --------------------------------------------------------------------------- CPU arm
-def cpu_reference(sample: str, steps: int, warmup: int):
+def cpu_reference(sample: str, steps: int, warmup: int, min_seconds: float = 10.0):
     """The reference's own CPU implementation cannot run here (100 % Julia, no `julia`
     binary in the image): the CPU arm is the C restatement in oracle/ with OpenMP on
-    every host core (kind "port").  A bounded sample of the same workload family."""
+    every host core (kind "port").  A bounded sample of the same workload family:
+    `steps` steps, extended up to `min_seconds` of CPU work (at most 200 steps)."""
     from oracle import oracle as O
     from sph_mountain_waves_b200 import cases
     nx, ny, nz = WORKLOADS[sample]
@@ -168,10 +177,9 @@ def cpu_reference(sample: str, steps: int, warmup: int):
     o.append(case.fields)
     o.create_cell_list()
     o.step("wcsph", warmup)
-    # bounded sample: at least `steps` steps and about 10 s of CPU work
     t0 = time.perf_counter()
     done = 0
-    while done < steps or (time.perf_counter() - t0 < 10.0 and done < 200):
+    while done < steps or (time.perf_counter() - t0 < min_seconds and done < 200):
         o.step("wcsph", 1)
         done += 1
     steps = done
@@ -187,8 +195,7 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps = max(1, min(args.steps, 5))
-    r = cpu_reference(args.cpu_sample, steps, min(args.warmup, 1))
+    r = cpu_reference(args.cpu_sample, args.steps, min(args.warmup, 1), min_seconds=0.0)
     line = {
         "impl": "reference", "metric": "particle-steps/s", "value": r["value"], "unit": "particle-steps/s",
         "n_gpus": args.gpus, "steps": r["steps"], "warmup": min(args.warmup, 1), "ms_per_step": r["ms_per_step"],
@@ -204,6 +211,41 @@ def run_reference(args):
 
 
 # --------------------------------------------------------------------------- GPU arm
+DUMP_FIELDS = ("h", "x", "m", "v", "rho_p", "rho", "type")   # the carried particle state
+DUMP_MAX_PARTICLES = 1 << 19   # x 12 float64 (index + 11 field components) = 48 MiB
+
+
+def dump_outputs(run, out_dir: str, rank: int, world: int):
+    """The particle state the timed steps left, as DIR/<field>.npy in global particle-index order
+    (DIR/index.npy holds the indices).  A run larger than DUMP_MAX_PARTICLES is sampled with a
+    fixed seed: the same particles for every build, so that two builds compare value for value."""
+    import torch.distributed as dist
+    n = run.n_global
+    if n <= DUMP_MAX_PARTICLES:
+        pick = np.arange(n, dtype=np.int64)
+    else:
+        pick = np.sort(np.random.default_rng(0).choice(n, DUMP_MAX_PARTICLES, replace=False))
+    want = np.zeros(n, dtype=bool)
+    want[pick] = True
+    gidx, fields = run.owned_fields(DUMP_FIELDS)
+    keep = want[gidx]
+    mine = (gidx[keep], {f: a[keep] for f, a in fields.items()})
+    parts = [mine]
+    if world > 1:
+        parts = [None] * world
+        dist.all_gather_object(parts, mine)
+    if rank != 0:
+        return
+    idx = np.concatenate([p[0] for p in parts])
+    order = np.argsort(idx, kind="stable")
+    assert np.array_equal(idx[order], pick), "the ranks do not own each sampled particle exactly once"
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    np.save(out / "index.npy", pick.astype(np.float64))
+    for f in DUMP_FIELDS:
+        np.save(out / f"{f}.npy", np.concatenate([p[1][f] for p in parts])[order].astype(np.float64))
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -266,6 +308,8 @@ def run_ours(args):
         ms = ev0.elapsed_time(ev1)
         launches = run.sys.launch_count() - l0
         rep = run.sys.timing_report()
+        if args.dump_outputs:
+            dump_outputs(run, args.dump_outputs, rank, world)
         # breakdown pass (not part of any reported throughput)
         nb = max(2, min(args.steps, 5))
         run.sys.timing(True)
