@@ -307,16 +307,29 @@ int sphmw_launch_count(sphmw_ctx *ctx, int64_t *n);
 /* ---- x-slab decomposition over the GPUs of one box (SURVEY.md §8e) ------------------
  * No reference equivalent: the reference is single-process (Threads.@threads,
  * src/core.jl:54-139).  A context created with slab_lo/slab_hi owns the global cell
- * columns [slab_lo, slab_hi) and keeps two ghost columns per side; it carries GLOBAL
- * particle indices so that neighbour order, and with it every FP64 sum, is the same
- * for any number of ranks.  Per step the host calls
+ * columns [slab_lo, slab_hi) and keeps two ghost columns per side (three with
+ * SPHMW_FLAG_GHOST3: the Hopkins schemes); it carries GLOBAL particle indices so that
+ * neighbour order, and with it every FP64 sum, is the same for any number of ranks.
+ * Per step the host calls
  *     sphmw_step_phase(ctx, "wcsph", 0)        accelerate! + move!
  *     sphmw_halo_pack -> transport -> sphmw_halo_unpack
  *     sphmw_step_phase(ctx, "wcsph", 1)        cell list, density pass, force pass + kick
- * (phases 2 and 3: the overlapped variant below).  A record is sphmw_halo_record_doubles() doubles; buffers are DEVICE pointers owned by
- * the caller (NULL = no neighbour on that side). */
+ * (phases 2 and 3: the overlapped variant below).  The same two phases step "hopkins",
+ * "hopkins_full" and "hopkins_total" (three ghost columns) and "aflow" (the adiabatic flow
+ * driver; phase 0 fails when an owned INFLOW particle would convert, because the successors'
+ * global indices need the library transport with the open box, below).  Host-driven steps do
+ * not renumber: a particle that leaves the global box is dropped and counted (counts[4]), which
+ * matches the reference's swap-from-end removal only while no particle leaves — the open box of
+ * the library transport replays it.
+ * A record is sphmw_halo_record_width(ctx) doubles: the base record of
+ * sphmw_halo_record_doubles() (13), or 17 for a context that holds the entropy S (the
+ * adiabatic flow driver: + S, P, T, theta).  The width is fixed at its first use (this query or
+ * the first pack/unpack/exchange; not sphmw_comm_init), so ask after the fields are uploaded: the
+ * answer is binding because buffers are sized by it.  Buffers are
+ * DEVICE pointers owned by the caller (NULL = no neighbour on that side). */
 int sphmw_step_phase(sphmw_ctx *ctx, const char *scheme, int32_t phase);
 int sphmw_halo_record_doubles(void);
+int sphmw_halo_record_width(sphmw_ctx *ctx, int32_t *doubles);
 /* counts: [0] records for the left neighbour, [1] for the right, [2],[3] migrants among
  * them, [4] particles that left the global box (dropped).  Blocks. */
 int sphmw_halo_pack(sphmw_ctx *ctx, double *dev_buf_left, double *dev_buf_right,
@@ -362,9 +375,14 @@ int sphmw_comm_info(sphmw_ctx *ctx, int64_t out[6]);
  * replays that loop on each rank, and sphmw_step uses the plain (non-overlapped) schedule.  Without
  * it (the default: walled configurations) a particle leaving the global box of a slab context is
  * dropped and counted (sphmw_comm_info out[4]), and an interior one fails the step loudly.
- * The open box also enables sphmw_step(ctx, "flow", n) on slabs: the inflow re-seeding of
- * isothermal_flow_witch.jl:175-186 numbers the new particles in the reference's order across ranks
- * (one all-gather of the converting indices per step). */
+ * The open box also enables sphmw_step(ctx, "flow" | "aflow", n) on slabs: the inflow re-seeding of
+ * isothermal_flow_witch.jl:175-186 / adiabatic_flow_witch.jl:197-208 numbers the new particles in the
+ * reference's order across ranks (one all-gather of the converting indices per step).  On such a
+ * context sphmw_flow_add_new_particles / sphmw_aflow_add_new_particles are collective and return the
+ * number added on all ranks, so the driver's operator-by-operator loop (sphmw_apply,
+ * add_new_particles, sphmw_create_cell_list) runs unchanged.  sphmw_step(ctx, "hopkins_total", n) needs
+ * three ghost columns (SPHMW_FLAG_GHOST3) and runs without the open box too: its walls move and fall
+ * (SURVEY quirk 10), and one that leaves the global box is then dropped and counted. */
 int sphmw_comm_open_box(sphmw_ctx *ctx, int32_t on);
 /* global particle index of every resident particle (physical order) */
 int sphmw_set_index(sphmw_ctx *ctx, const int64_t *global_idx, int64_t n);

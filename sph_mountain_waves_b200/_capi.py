@@ -118,6 +118,7 @@ _SIGS = {
     "sphmw_launch_count": (C.c_int, [_P, C.POINTER(C.c_int64)]),
     "sphmw_step_phase": (C.c_int, [_P, C.c_char_p, C.c_int32]),
     "sphmw_halo_record_doubles": (C.c_int, []),
+    "sphmw_halo_record_width": (C.c_int, [_P, C.POINTER(C.c_int32)]),
     "sphmw_halo_pack": (C.c_int, [_P, C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(C.c_int64)]),
     "sphmw_halo_pack_begin": (C.c_int, [_P, C.c_void_p, C.c_void_p, C.c_int64]),
     "sphmw_halo_pack_finish": (C.c_int, [_P, C.c_int64, C.POINTER(C.c_int64)]),

@@ -14,17 +14,19 @@
 // locally and no second exchange is needed before the force pass.
 #include <string.h>
 
+#include "halo_record.cuh"
 #include "sphmw_internal.h"
 
 // cf: only the particles that sat in the selected columns BEFORE the drift (cellx is the
 // column of the last cell list) are looked at — the overlapped step packs the edge columns
 // while the interior is still in the force pass; cf.on == 0 looks at everybody.
-template <int DIM>
+template <int DIM, int KIND>
 __global__ void k_halo_pack(Fields f, const uint32_t *__restrict__ idx, uint32_t *__restrict__ tag,
                             int64_t n, Grid g, int has_left, int has_right, double *buf_l,
                             double *buf_r, uint32_t cap, uint32_t *counters,
                             const uint32_t *__restrict__ cellx, ColFilter cf, uint32_t *__restrict__ lost_list,
                             uint32_t lost_cap, int carry_a) {
+    constexpr int ROWS = halo_record_rows(KIND);
     int64_t p = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (p >= n) return;
     if (cf.on && !col_selected(cf, (int)cellx[p])) return;
@@ -65,67 +67,29 @@ __global__ void k_halo_pack(Fields f, const uint32_t *__restrict__ idx, uint32_t
     to_l = to_l && has_left;
     to_r = to_r && has_right;
     if (!to_l && !to_r) return;
-    double rec[HALO_RECORD];
-    rec[0] = x;
-    rec[1] = y;
-    rec[2] = z;
-    rec[3] = f.s[S_V0][p];
-    rec[4] = f.s[S_V1][p];
-    rec[5] = DIM == 3 ? f.s[S_V2][p] : 0.0;
-    rec[6] = f.s[S_M][p];
-    rec[7] = f.s[S_H][p];
-    // rows 8/9: rho, rho' — or, for the pressure-entropy (Hopkins) drivers, the entropy functions A and
-    // A_bg, which are carried state there (densities are recomputed by the receiver either way)
-    rec[8] = carry_a ? f.s[S_A][p] : f.s[S_RHO][p];
-    rec[9] = carry_a ? (carry_a > 1 ? f.s[S_A_BG][p] : 0.0) : f.s[S_RHO_P][p];
-    rec[10] = f.s[S_TYPE][p];
-    rec[11] = (double)idx[p];
-    rec[12] = kind;
+    double rec[ROWS];
+    halo_record_pack<DIM, KIND>(f, idx, p, x, y, z, kind, carry_a, rec);  // halo_record.cuh
     if (to_l) {
         uint32_t s = atomicAdd(&counters[0], 1u);
         if (kind == HALO_KIND_MIGRANT) atomicAdd(&counters[2], 1u);
         if (s < cap)
-            for (int k = 0; k < HALO_RECORD; ++k) buf_l[(size_t)s * HALO_RECORD + k] = rec[k];
+            for (int k = 0; k < ROWS; ++k) buf_l[(size_t)s * ROWS + k] = rec[k];
     }
     if (to_r) {
         uint32_t s = atomicAdd(&counters[1], 1u);
         if (kind == HALO_KIND_MIGRANT) atomicAdd(&counters[3], 1u);
         if (s < cap)
-            for (int k = 0; k < HALO_RECORD; ++k) buf_r[(size_t)s * HALO_RECORD + k] = rec[k];
+            for (int k = 0; k < ROWS; ++k) buf_r[(size_t)s * ROWS + k] = rec[k];
     }
 }
 
-template <int DIM>
+template <int DIM, int KIND>
 __global__ void k_halo_unpack(Fields f, uint32_t *__restrict__ idx, uint32_t *__restrict__ tag,
                               int64_t first, const double *__restrict__ buf, int64_t cnt, int carry_a) {
     int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (t >= cnt) return;
-    const double *rec = buf + (size_t)t * HALO_RECORD;
-    int64_t p = first + t;
-    f.s[S_X0][p] = rec[0];
-    f.s[S_X1][p] = rec[1];
-    if (DIM == 3) f.s[S_X2][p] = rec[2];
-    f.s[S_V0][p] = rec[3];
-    f.s[S_V1][p] = rec[4];
-    if (DIM == 3) f.s[S_V2][p] = rec[5];
-    f.s[S_M][p] = rec[6];
-    f.s[S_H][p] = rec[7];
-    if (carry_a) {
-        f.s[S_A][p] = rec[8];
-        if (carry_a > 1) f.s[S_A_BG][p] = rec[9];
-    } else {
-        f.s[S_RHO][p] = rec[8];
-        f.s[S_RHO_P][p] = rec[9];
-    }
-    f.s[S_TYPE][p] = rec[10];
-    idx[p] = (uint32_t)rec[11];
-    tag[p] = rec[12] == HALO_KIND_MIGRANT ? TAG_OWNED : TAG_GHOST;
-    // accumulators of the op-by-op schemes: the sender's move! / find_pressure! left them zero
-    // (isothermal_flow_witch.jl:157,205), the slot here may hold anything
-    if (f.s[S_DRHO]) f.s[S_DRHO][p] = 0.0;
-    if (f.s[S_DV0]) f.s[S_DV0][p] = 0.0;
-    if (f.s[S_DV1]) f.s[S_DV1][p] = 0.0;
-    if (DIM == 3 && f.s[S_DV2]) f.s[S_DV2][p] = 0.0;
+    const double *rec = buf + (size_t)t * halo_record_rows(KIND);
+    halo_record_unpack<DIM, KIND>(f, idx, tag, first + t, rec, carry_a);  // halo_record.cuh
 }
 
 static const int CARRIED[] = {S_X0, S_X1, S_X2, S_V0, S_V1, S_V2, S_M, S_H, S_RHO, S_RHO_P, S_TYPE};
@@ -136,7 +100,25 @@ static int carry_a(const sphmw_ctx *c) {
     return c->allocated[S_A_BG] ? 2 : 1;
 }
 
-static int ensure_carried(sphmw_ctx *c) {
+// The record kind of a context's halo exchange (halo_record.cuh): ADIABATIC when the context holds the
+// entropy S (the adiabatic flow driver), BASE otherwise.  Fixed at its first use: the first pack, unpack
+// or library-transport exchange, or sphmw_halo_record_width — a caller sizes its record buffers by that
+// answer, so a later pack must not write wider records into them.  Records of another width are never
+// sent; a context whose fields would change the kind later fails instead.  (sphmw_comm_init does not
+// decide it: a communicator may exist before the fields are uploaded.)
+int sphmw_halo_kind(sphmw_ctx *c, int *kind) {
+    const int want = c->allocated[S_ENT] ? HALO_REC_ADIABATIC : HALO_REC_BASE;
+    if (c->halo_kind < 0) c->halo_kind = want;
+    if (c->halo_kind != want) {
+        sphmw_set_error("halo: the context's fields now call for %d-row records, its exchange was set up with %d rows",
+                        halo_record_rows(want), halo_record_rows(c->halo_kind));
+        return SPHMW_E_STATE;
+    }
+    *kind = want;
+    return SPHMW_OK;
+}
+
+static int ensure_carried(sphmw_ctx *c, int kind) {
     for (int s : CARRIED) {
         if (c->grid.dim == 2 && (s == S_X2 || s == S_V2)) continue;
         TRY(sphmw_ensure_slot(c, s));
@@ -144,22 +126,49 @@ static int ensure_carried(sphmw_ctx *c) {
     }
     for (int s : {S_A, S_A_BG})
         if (c->allocated[s] && c->stale[s]) { sphmw_set_error("halo: carried field is stale"); return SPHMW_E_STATE; }
+    if (kind == HALO_REC_ADIABATIC)
+        for (int s : {S_ENT, S_P, S_T, S_TH}) {
+            TRY(sphmw_ensure_slot(c, s));
+            if (c->stale[s]) { sphmw_set_error("halo: carried field is stale"); return SPHMW_E_STATE; }
+        }
     return SPHMW_OK;
 }
 
+// the base record (contexts without the entropy S); sphmw_halo_record_width gives a context's own
 extern "C" int sphmw_halo_record_doubles(void) { return HALO_RECORD; }
 
-// row 0 of a message (slab_comm.cu): {records, migrants among them}; the records follow
-__global__ void k_halo_header(const uint32_t *__restrict__ counters, double *msg_l, double *msg_r) {
+extern "C" int sphmw_halo_record_width(sphmw_ctx *c, int32_t *doubles) {
+    if (!c || !doubles) { sphmw_set_error("null argument"); return SPHMW_E_INVALID; }
+    int kind = 0;
+    TRY(sphmw_halo_kind(c, &kind));
+    *doubles = halo_record_rows(kind);
+    return SPHMW_OK;
+}
+
+// row 0 of a message (slab_comm.cu): {records, migrants among them, record width}; the records follow
+__global__ void k_halo_header(const uint32_t *__restrict__ counters, double *msg_l, double *msg_r, int width) {
     if (threadIdx.x == 0 && msg_l) {
         msg_l[0] = (double)counters[0];
         msg_l[1] = (double)counters[2];
+        msg_l[2] = (double)width;
     }
     if (threadIdx.x == 1 && msg_r) {
         msg_r[0] = (double)counters[1];
         msg_r[1] = (double)counters[3];
+        msg_r[2] = (double)width;
     }
 }
+
+#define HALO_LAUNCH(KERNEL, BLOCKS, ...)                                                                  \
+    do {                                                                                              \
+        if (c->grid.dim == 2) {                                                                       \
+            if (kind == HALO_REC_ADIABATIC) KERNEL<2, HALO_REC_ADIABATIC><<<BLOCKS, 256, 0, c->stream>>>(__VA_ARGS__); \
+            else KERNEL<2, HALO_REC_BASE><<<BLOCKS, 256, 0, c->stream>>>(__VA_ARGS__);                \
+        } else {                                                                                      \
+            if (kind == HALO_REC_ADIABATIC) KERNEL<3, HALO_REC_ADIABATIC><<<BLOCKS, 256, 0, c->stream>>>(__VA_ARGS__); \
+            else KERNEL<3, HALO_REC_BASE><<<BLOCKS, 256, 0, c->stream>>>(__VA_ARGS__);                \
+        }                                                                                             \
+    } while (0)
 
 // enqueue: classify + pack (all particles, or the edge columns of an overlapped step out of the
 // alt buffers), then read the counters back asynchronously and mark the point with an event
@@ -167,7 +176,9 @@ __global__ void k_halo_header(const uint32_t *__restrict__ counters, double *msg
 // these messages (the records themselves start one row further, at dev_buf_*)
 static int pack_enqueue(sphmw_ctx *c, double *dev_buf_left, double *dev_buf_right, int64_t cap_records,
                         bool edge_only, double *msg_left = nullptr, double *msg_right = nullptr) {
-    TRY(ensure_carried(c));
+    int kind = 0;
+    TRY(sphmw_halo_kind(c, &kind));
+    TRY(ensure_carried(c, kind));
     // what the next cell-list build will find dead: last exchange's ghosts and migrants, plus
     // the particles this pack is about to drop (added by pack_collect)
     c->slab_dead_expected = c->n - c->n_owned;
@@ -183,20 +194,15 @@ static int pack_enqueue(sphmw_ctx *c, double *dev_buf_left, double *dev_buf_righ
             cf = sphmw_slab_cols(c).edge;
         }
         TIMED(c, "halo_pack");
-        if (c->grid.dim == 2)
-            k_halo_pack<2><<<grid_for(c->n, 256), 256, 0, c->stream>>>(
-                view, c->idx, c->tag, c->n, c->grid, has_left, has_right, dev_buf_left,
-                dev_buf_right, (uint32_t)cap_records, c->halo_counters, c->cellx, cf, c->lost_list, SLAB_LOST_CAP, carry_a(c));
-        else
-            k_halo_pack<3><<<grid_for(c->n, 256), 256, 0, c->stream>>>(
-                view, c->idx, c->tag, c->n, c->grid, has_left, has_right, dev_buf_left,
-                dev_buf_right, (uint32_t)cap_records, c->halo_counters, c->cellx, cf, c->lost_list, SLAB_LOST_CAP, carry_a(c));
+        HALO_LAUNCH(k_halo_pack, grid_for(c->n, 256), view, c->idx, c->tag, c->n, c->grid, has_left, has_right, dev_buf_left,
+                    dev_buf_right, (uint32_t)cap_records, c->halo_counters, c->cellx, cf, c->lost_list, SLAB_LOST_CAP,
+                    carry_a(c));
         CUDA_TRY(cudaGetLastError());
     }
     if (c->lost_list)  // word 0 of the list: how many particles this pack dropped
         CUDA_TRY(cudaMemcpyAsync(c->lost_list, c->halo_counters + 4, sizeof(uint32_t), cudaMemcpyDeviceToDevice, c->stream));
     if (msg_left || msg_right) {
-        k_halo_header<<<1, 32, 0, c->stream>>>(c->halo_counters, msg_left, msg_right);
+        k_halo_header<<<1, 32, 0, c->stream>>>(c->halo_counters, msg_left, msg_right, halo_record_rows(kind));
         c->launches += 1;
     }
     TRY(sphmw_publish_words(c, c->halo_counters, c->h_halo_counters, 8, c->stream));
@@ -205,7 +211,10 @@ static int pack_enqueue(sphmw_ctx *c, double *dev_buf_left, double *dev_buf_righ
     return SPHMW_OK;
 }
 int sphmw_halo_pack_enqueue(sphmw_ctx *c, double *msg_left, double *msg_right, int64_t cap_records, bool edge_only) {
-    return pack_enqueue(c, msg_left ? msg_left + HALO_RECORD : nullptr, msg_right ? msg_right + HALO_RECORD : nullptr,
+    int kind = 0;
+    TRY(sphmw_halo_kind(c, &kind));
+    const int W = halo_record_rows(kind);
+    return pack_enqueue(c, msg_left ? msg_left + W : nullptr, msg_right ? msg_right + W : nullptr,
                         cap_records, edge_only, msg_left, msg_right);
 }
 
@@ -286,15 +295,12 @@ extern "C" int sphmw_halo_unpack(sphmw_ctx *c, const double *dev_buf, int64_t co
                         (long long)count, (long long)c->cap);
         return SPHMW_E_CAPACITY;
     }
-    TRY(ensure_carried(c));
+    int kind = 0;
+    TRY(sphmw_halo_kind(c, &kind));
+    TRY(ensure_carried(c, kind));
     {
         TIMED(c, "halo_unpack");
-        if (c->grid.dim == 2)
-            k_halo_unpack<2><<<grid_for(count, 256), 256, 0, c->stream>>>(
-                c->cur, c->idx, c->tag, c->n, dev_buf, count, carry_a(c));
-        else
-            k_halo_unpack<3><<<grid_for(count, 256), 256, 0, c->stream>>>(
-                c->cur, c->idx, c->tag, c->n, dev_buf, count, carry_a(c));
+        HALO_LAUNCH(k_halo_unpack, grid_for(count, 256), c->cur, c->idx, c->tag, c->n, dev_buf, count, carry_a(c));
         CUDA_TRY(cudaGetLastError());
     }
     c->n += count;

@@ -750,8 +750,9 @@ __global__ void k_flow_spawn_list(Fields f, Params c, uint32_t *__restrict__ idx
     tag[s] = TAG_OWNED;
 }
 // collect: list[0] = count, list[1..] = global indices, pos[k] = physical position (device arrays)
-int sphmw_flow_collect_slab(sphmw_ctx *c, uint32_t *list, uint32_t *pos, uint32_t cap) {
+int sphmw_flow_collect_slab(sphmw_ctx *c, uint32_t *list, uint32_t *pos, uint32_t cap, bool adiabatic) {
     TRY(need_slots(c, SL(S_X0, S_V0, S_TYPE, S_RHO, S_M, S_P, S_TH), SL(S_X0, S_V0, S_TYPE, S_RHO, S_M, S_P, S_TH)));
+    if (adiabatic) TRY(need_slots(c, SL(S_T, S_ENT), SL(S_T, S_ENT)));
     CUDA_TRY(cudaMemsetAsync(list, 0, sizeof(uint32_t), c->stream));
     if (c->n == 0) return SPHMW_OK;
     TIMED(c, "flow.flag_inflow");
@@ -761,7 +762,7 @@ int sphmw_flow_collect_slab(sphmw_ctx *c, uint32_t *list, uint32_t *pos, uint32_
     return SPHMW_OK;
 }
 // build m successors at the end of the resident set: pos[k] converts, its successor gets new_idx[k]
-int sphmw_flow_spawn_slab(sphmw_ctx *c, const uint32_t *pos, const uint32_t *new_idx, int m) {
+int sphmw_flow_spawn_slab(sphmw_ctx *c, const uint32_t *pos, const uint32_t *new_idx, int m, bool adiabatic) {
     if (m <= 0) return SPHMW_OK;
     const int64_t n = c->n;
     if (n + m > c->cap) {
@@ -771,8 +772,15 @@ int sphmw_flow_spawn_slab(sphmw_ctx *c, const uint32_t *pos, const uint32_t *new
     for (int s = 0; s < NSLOT; ++s)  // every other field of a new particle is the constructor's zero
         if (c->allocated[s]) CUDA_TRY(cudaMemsetAsync(c->cur.s[s] + n, 0, sizeof(double) * m, c->stream));
     TIMED(c, "flow.spawn_inflow");
-    if (c->grid.dim == 2) k_flow_spawn_list<2, false><<<grid_for(m, 128), 128, 0, c->stream>>>(c->cur, c->prm, c->idx, c->tag, n, pos, new_idx, m);
-    else k_flow_spawn_list<3, false><<<grid_for(m, 128), 128, 0, c->stream>>>(c->cur, c->prm, c->idx, c->tag, n, pos, new_idx, m);
+#define SPAWN_LIST(D, A) k_flow_spawn_list<D, A><<<grid_for(m, 128), 128, 0, c->stream>>>(c->cur, c->prm, c->idx, c->tag, n, pos, new_idx, m)
+    if (c->grid.dim == 2) {
+        if (adiabatic) SPAWN_LIST(2, true);
+        else SPAWN_LIST(2, false);
+    } else {
+        if (adiabatic) SPAWN_LIST(3, true);
+        else SPAWN_LIST(3, false);
+    }
+#undef SPAWN_LIST
     CUDA_TRY(cudaGetLastError());
     c->n = n + m;
     c->n_owned += m;
@@ -782,7 +790,16 @@ int sphmw_flow_spawn_slab(sphmw_ctx *c, const uint32_t *pos, const uint32_t *new
 
 int sphmw_flow_add_particles(sphmw_ctx *c, int64_t *n_added, bool adiabatic) {
     if (n_added) *n_added = 0;
-    if (c->slab_lo >= 0) { sphmw_set_error("add_new_particles: whole-domain contexts only"); return SPHMW_E_STATE; }
+    if (c->slab_lo >= 0) {
+        // the successors' global indices follow from the converting particles of ALL ranks: collective
+        // (slab_comm.cu), through the library transport with the open box
+        if (!c->comm) {
+            sphmw_set_error("add_new_particles: a slab context re-seeds its inflow through the library transport "
+                            "(sphmw_comm_init + sphmw_comm_open_box)");
+            return SPHMW_E_STATE;
+        }
+        return sphmw_comm_add_new_particles(c, n_added, adiabatic);
+    }
     const int64_t n = c->n;
     if (n == 0) return SPHMW_OK;
     TRY(need_slots(c, SL(S_X0, S_V0, S_TYPE, S_RHO, S_M, S_P, S_TH), SL(S_X0, S_V0, S_TYPE, S_RHO, S_M, S_P, S_TH)));
@@ -1186,7 +1203,71 @@ static int step_wcsph_overlap_b(sphmw_ctx *c) {
     return SPHMW_OK;
 }
 
+// hopkins_total_witch.jl:283-308 on a slab context: compute_pressure! reads the neighbours' NEW smoothing
+// length, as in the other Hopkins drivers, so the context needs three ghost columns.  The base halo
+// record with A in row 8 carries everything: rho, P, T and theta are recomputed for every particle type
+// before they are read (U_ht_reset_density, U_ht_reset_pressure/finalize_pressure, U_ht_find_temperature,
+// U_ht_find_pot_temp are not type-gated), and Dv is zero after accelerate!.  Walls move and feel gravity in
+// this driver (SURVEY quirk 10): one that leaves the global box is dropped and counted as on any walled
+// configuration, or renumbered like the reference with the open box (slab_comm.cu).
+static int step_hopkins_total_phase(sphmw_ctx *c, int phase) {
+    if (c->slab_lo >= 0 && c->grid.ghost < 3) {
+        sphmw_set_error("the Hopkins schemes need three ghost columns on a slab context (SPHMW_FLAG_GHOST3)");
+        return SPHMW_E_STATE;
+    }
+    if (phase == 0) return apply_seq(c, {"hopkins_total.accelerate", "hopkins_total.move"});
+    if (phase == 1)
+        return apply_seq(c, {"create_cell_list", "hopkins_total.reset_density", "wcsph.compute_density",
+                             "wcsph.update_smoothing", "hopkins_total.reset_pressure", "hopkins.compute_pressure",
+                             "hopkins_total.finalize_pressure", "hopkins_total.find_temperature",
+                             "hopkins_total.find_pot_temp", "hopkins_total.balance_of_momentum",
+                             "hopkins_total.accelerate"});
+    sphmw_set_error("step_phase: the Hopkins schemes run the plain schedule (phases 0 and 1)");
+    return SPHMW_E_INVALID;
+}
+
+// adiabatic_flow_witch.jl:231-243 on a slab context driven by the caller's transport.  add_new_particles!
+// numbers the successors across ranks, which only the library transport can do (sphmw_comm_open_box):
+// phase 0 refuses a step in which an owned INFLOW particle would convert instead of skipping it.
+static int step_aflow_phase(sphmw_ctx *c, int phase) {
+    if (c->slab_lo < 0) {
+        sphmw_set_error("step_phase 'aflow': slab contexts only (a whole-domain context steps with sphmw_step)");
+        return SPHMW_E_STATE;
+    }
+    if (phase == 0) {
+        TRY(apply_seq(c, {"flow.accelerate", "aflow.move"}));
+        TRY(need_slots(c, SL(S_X0, S_TYPE), SL()));
+        uint32_t *count = c->rank;  // scratch of the cell-list build, free between builds
+        CUDA_TRY(cudaMemsetAsync(count, 0, sizeof(uint32_t), c->stream));
+        if (c->n > 0) {
+            TIMED(c, "flow.flag_inflow");
+            if (c->grid.dim == 2) k_flow_collect<2><<<grid_for(c->n, 256), 256, 0, c->stream>>>(c->cur, c->prm, c->idx, c->tag, c->n, count, nullptr, 0);
+            else k_flow_collect<3><<<grid_for(c->n, 256), 256, 0, c->stream>>>(c->cur, c->prm, c->idx, c->tag, c->n, count, nullptr, 0);
+            CUDA_TRY(cudaGetLastError());
+        }
+        uint32_t converting = 0;
+        CUDA_TRY(cudaMemcpyAsync(&converting, count, sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+        CUDA_TRY(cudaStreamSynchronize(c->stream));
+        if (converting) {
+            sphmw_set_error("step_phase 'aflow': %u INFLOW particle(s) of this rank convert in this step; their successors "
+                            "are numbered across ranks, which needs the library transport with the open box "
+                            "(sphmw_comm_init, sphmw_comm_open_box, sphmw_step)", converting);
+            return SPHMW_E_STATE;
+        }
+        return SPHMW_OK;
+    }
+    if (phase == 1) {
+        TRY(sphmw_build_cell_list(c, nullptr));
+        return apply_seq(c, {"+aflow.find_density", "aflow.find_s", "aflow.find_pressure", "aflow.entropy_production",
+                             "flow.internal_force", "flow.accelerate"});
+    }
+    sphmw_set_error("step_phase: the 'aflow' scheme runs the plain schedule (phases 0 and 1)");
+    return SPHMW_E_INVALID;
+}
+
 int sphmw_step_scheme_phase(sphmw_ctx *c, const char *scheme, int phase) {
+    if (!strcmp(scheme, "hopkins_total")) return step_hopkins_total_phase(c, phase);
+    if (!strcmp(scheme, "aflow")) return step_aflow_phase(c, phase);
     if (!strcmp(scheme, "hopkins") || !strcmp(scheme, "hopkins_full")) {
         // plain schedule only: kick + drift | (the caller's halo exchange) | sort + three pair passes
         if (phase == 0) return step_wcsph_fused_pre(c);
@@ -1197,7 +1278,8 @@ int sphmw_step_scheme_phase(sphmw_ctx *c, const char *scheme, int phase) {
         return SPHMW_E_INVALID;
     }
     if (strcmp(scheme, "wcsph")) {
-        sphmw_set_error("step_phase: only the fused 'wcsph' and 'hopkins'/'hopkins_full' schemes run on slabs");
+        sphmw_set_error("step_phase: only the 'wcsph', 'hopkins', 'hopkins_full', 'hopkins_total' and 'aflow' schemes "
+                        "run on slabs");
         return SPHMW_E_UNSUPPORTED_OP;
     }
     switch (phase) {

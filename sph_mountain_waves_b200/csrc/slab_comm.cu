@@ -4,9 +4,10 @@
 // the reference's caller is one (src/core.jl:125-142) — steps a slab context with the very calls
 // it uses on one GPU.
 //
-// One exchange = ONE ncclGroup per step.  A message is a fixed number of rows of HALO_RECORD
-// doubles agreed between the two ranks; row 0 is written on the device by the pack
-// ({records, migrants}), so no count has to travel first and the sender's host never has to
+// One exchange = ONE ncclGroup per step.  A message is a fixed number of rows of `width` doubles (the
+// context's halo record, halo_record.cuh: 13, or 17 for the adiabatic flow driver) agreed between the
+// two ranks; row 0 is written on the device by the pack ({records, migrants, width}; the receiver
+// checks the width against its own), so no count has to travel first and the sender's host never has to
 // know it before the send is queued.  The sizes are agreed once (a header-only round at the first
 // exchange: count * 1.12 + 1024 rows) and renegotiated, with one extra blocking round, only when a
 // count outgrows them.  Per step the host waits once — for the two received headers, which arrive
@@ -24,6 +25,7 @@
 #include <utility>
 #include <vector>
 
+#include "halo_record.cuh"
 #include "sphmw_internal.h"
 
 struct NcclApi {
@@ -90,6 +92,7 @@ struct SlabComm {
     int peer[2] = {-1, -1};
     cudaStream_t stream = nullptr;  // high priority: the transfer runs beside the interior force pass
     int64_t cap = 0;                // records a message buffer holds (+ the header row)
+    int width = 0;                  // doubles per row: the context's record width; 0 until the first exchange
     double *send[2] = {nullptr, nullptr}, *recv[2] = {nullptr, nullptr};
     int64_t send_rows[2] = {0, 0}, recv_rows[2] = {0, 0};  // agreed message sizes (0: not yet)
     double *h_head = nullptr;       // pinned: the two received headers
@@ -177,20 +180,33 @@ extern "C" int sphmw_comm_init(sphmw_ctx *c, int32_t rank, int32_t world, const 
         CUDA_TRY(cudaDeviceGetStreamPriorityRange(&lo, &hi));
         CUDA_TRY(cudaStreamCreateWithPriority(&m->stream, cudaStreamNonBlocking, hi));
         CUDA_TRY(cudaEventCreateWithFlags(&m->recv_event, cudaEventDisableTiming));
-        CUDA_TRY(cudaMallocHost(&m->h_head, sizeof(double) * 2 * HALO_RECORD));
-        for (int s = 0; s < 2; ++s)
-            if (m->has[s]) {
-                const size_t bytes = sizeof(double) * HALO_RECORD * (size_t)(m->cap + 1);
-                CUDA_TRY(cudaMalloc(&m->send[s], bytes));
-                CUDA_TRY(cudaMalloc(&m->recv[s], bytes));
-                CUDA_TRY(cudaMemsetAsync(m->send[s], 0, bytes, c->stream));
-                CUDA_TRY(cudaMemsetAsync(m->recv[s], 0, bytes, c->stream));
-            }
-        CUDA_TRY(cudaStreamSynchronize(c->stream));
         return SPHMW_OK;
     }();
     if (rc != SPHMW_OK) sphmw_comm_free(c);
     return rc;
+}
+
+// The message buffers and the pinned header rows, made at the first exchange: the record width follows
+// from the fields the context holds (halo.cu sphmw_halo_kind), and a caller may create the communicator
+// before it uploads them (the Julia shim does: sphmw_create, sphmw_comm_init, then the upload).
+static int comm_buffers(sphmw_ctx *c) {
+    SlabComm *m = c->comm;
+    if (m->width > 0) return SPHMW_OK;
+    int kind = 0;
+    TRY(sphmw_halo_kind(c, &kind));
+    const int width = halo_record_rows(kind);
+    CUDA_TRY(cudaMallocHost(&m->h_head, sizeof(double) * 2 * width));
+    for (int s = 0; s < 2; ++s)
+        if (m->has[s]) {
+            const size_t bytes = sizeof(double) * width * (size_t)(m->cap + 1);
+            CUDA_TRY(cudaMalloc(&m->send[s], bytes));
+            CUDA_TRY(cudaMalloc(&m->recv[s], bytes));
+            CUDA_TRY(cudaMemsetAsync(m->send[s], 0, bytes, c->stream));
+            CUDA_TRY(cudaMemsetAsync(m->recv[s], 0, bytes, c->stream));
+        }
+    CUDA_TRY(cudaStreamSynchronize(c->stream));
+    m->width = width;
+    return SPHMW_OK;
 }
 
 extern "C" int sphmw_comm_info(sphmw_ctx *c, int64_t out[6]) {
@@ -215,14 +231,14 @@ static int comm_round(sphmw_ctx *c, const int64_t srows[2], const int64_t rrows[
     for (int s = 0; s < 2; ++s) {
         if (!m->has[s]) continue;
         if (srows[s] > 0)
-            NCCL_TRY(g_nccl.Send(m->send[s], (size_t)srows[s] * HALO_RECORD, ncclDouble, m->peer[s], m->comm, m->stream));
+            NCCL_TRY(g_nccl.Send(m->send[s], (size_t)srows[s] * m->width, ncclDouble, m->peer[s], m->comm, m->stream));
         if (rrows[s] > 0)
-            NCCL_TRY(g_nccl.Recv(m->recv[s], (size_t)rrows[s] * HALO_RECORD, ncclDouble, m->peer[s], m->comm, m->stream));
+            NCCL_TRY(g_nccl.Recv(m->recv[s], (size_t)rrows[s] * m->width, ncclDouble, m->peer[s], m->comm, m->stream));
     }
     NCCL_TRY(g_nccl.GroupEnd());
     for (int s = 0; s < 2; ++s)
         if (m->has[s] && rrows[s] > 0)  // (a kernel store, not a copy-engine transfer: see sphmw_publish_words)
-            TRY(sphmw_publish_words(c, (const uint32_t *)m->recv[s], (uint32_t *)(m->h_head + s * HALO_RECORD), 2 * HALO_RECORD,
+            TRY(sphmw_publish_words(c, (const uint32_t *)m->recv[s], (uint32_t *)(m->h_head + s * m->width), 2 * m->width,
                                     m->stream));
     CUDA_TRY(cudaEventRecord(m->recv_event, m->stream));
     return SPHMW_OK;
@@ -245,8 +261,14 @@ static int comm_transfer_and_unpack(sphmw_ctx *c) {
     int64_t in_count[2] = {0, 0}, in_migr[2] = {0, 0};
     for (int s = 0; s < 2; ++s)
         if (m->has[s]) {
-            in_count[s] = (int64_t)m->h_head[s * HALO_RECORD];
-            in_migr[s] = (int64_t)m->h_head[s * HALO_RECORD + 1];
+            const double *head = m->h_head + s * m->width;
+            if (head[2] != (double)m->width) {
+                sphmw_set_error("halo message from rank %d has %g-double records, this rank's have %d (the ranks hold "
+                                "different particle fields)", m->peer[s], head[2], m->width);
+                return SPHMW_E_STATE;
+            }
+            in_count[s] = (int64_t)head[0];
+            in_migr[s] = (int64_t)head[1];
             if (in_count[s] > m->cap) {
                 sphmw_set_error("halo message of %lld records exceeds the buffer capacity %lld", (long long)in_count[s],
                                 (long long)m->cap);
@@ -279,7 +301,7 @@ static int comm_transfer_and_unpack(sphmw_ctx *c) {
     // the main stream appends what arrived (the transfer is complete: the host has waited for it)
     for (int s = 0; s < 2; ++s)
         if (m->has[s] && in_count[s] > 0)
-            TRY(sphmw_halo_unpack(c, m->recv[s] + HALO_RECORD, in_count[s], in_migr[s]));
+            TRY(sphmw_halo_unpack(c, m->recv[s] + m->width, in_count[s], in_migr[s]));
     return SPHMW_OK;
 }
 
@@ -387,17 +409,19 @@ static int comm_renumber_lost(sphmw_ctx *c) {
     return SPHMW_OK;
 }
 
-// ≙ add_new_particles!(sys) (isothermal_flow_witch.jl:175-186) on a slab decomposition.  The
+// ≙ add_new_particles!(sys) (isothermal_flow_witch.jl:175-186; adiabatic_flow_witch.jl:197-208 with
+// `adiabatic`) on a slab decomposition.  The
 // reference's loop runs over sys.particles in index order and appends one successor per converting
 // INFLOW particle, so successor k gets index N + k where k counts the converting particles of ALL
 // ranks with a smaller index: every rank contributes its list (one all-gather per step), the merged
 // list is sorted on every host, and each rank builds the successors of its own particles with the
-// indices that order gives them.
-static int comm_flow_spawn(sphmw_ctx *c) {
+// indices that order gives them.  *n_added (optional): successors made on all ranks.
+static int comm_flow_spawn(sphmw_ctx *c, bool adiabatic, int64_t *n_added = nullptr) {
     SlabComm *m = c->comm;
+    if (n_added) *n_added = 0;
     if (m->n_global < 0) TRY(comm_count_global(c));
     const size_t block = 1 + SLAB_LOST_CAP;
-    TRY(sphmw_flow_collect_slab(c, m->conv_list, m->conv_pos, SLAB_LOST_CAP));
+    TRY(sphmw_flow_collect_slab(c, m->conv_list, m->conv_pos, SLAB_LOST_CAP, adiabatic));
     CUDA_TRY(cudaEventRecord(c->pack_event, c->stream));
     CUDA_TRY(cudaStreamWaitEvent(m->stream, c->pack_event, 0));
     NCCL_TRY(g_nccl.AllGather(m->conv_list, m->gather_dev, block, ncclUint32, m->comm, m->stream));
@@ -426,14 +450,28 @@ static int comm_flow_spawn(sphmw_ctx *c) {
         }
         CUDA_TRY(cudaMemcpyAsync(m->conv_pos + SLAB_LOST_CAP, m->h_conv + SLAB_LOST_CAP, sizeof(uint32_t) * k,
                                  cudaMemcpyHostToDevice, c->stream));
-        TRY(sphmw_flow_spawn_slab(c, m->conv_pos, m->conv_pos + SLAB_LOST_CAP, k));
+        TRY(sphmw_flow_spawn_slab(c, m->conv_pos, m->conv_pos + SLAB_LOST_CAP, k, adiabatic));
     }
     m->n_global += (int64_t)all.size();
+    if (n_added) *n_added = (int64_t)all.size();
     return SPHMW_OK;
+}
+
+// sphmw_flow_add_new_particles / sphmw_aflow_add_new_particles on a slab context: collective, the same
+// spawn as sphmw_step(ctx, "flow" | "aflow", n); *n_added counts the particles added on all ranks
+int sphmw_comm_add_new_particles(sphmw_ctx *c, int64_t *n_added, bool adiabatic) {
+    if (!c->comm->open_box) {
+        sphmw_set_error("add_new_particles: inflow re-seeding renumbers particles across ranks; call "
+                        "sphmw_comm_open_box first");
+        return SPHMW_E_STATE;
+    }
+    if (c->overlap_stage != 0) { sphmw_set_error("add_new_particles: an overlapped step is in flight"); return SPHMW_E_STATE; }
+    return comm_flow_spawn(c, adiabatic, n_added);
 }
 
 static int comm_exchange_all(sphmw_ctx *c) {
     SlabComm *m = c->comm;
+    TRY(comm_buffers(c));
     if (m->open_box && m->n_global < 0) TRY(comm_count_global(c));
     TRY(sphmw_halo_pack_enqueue(c, m->send[0], m->send[1], m->cap, false));
     TRY(comm_transfer_and_unpack(c));
@@ -453,32 +491,41 @@ int sphmw_comm_create_cell_list(sphmw_ctx *c, int64_t *n_alive) {
 // packed first and their records travel while the interior columns are in the force pass.
 int sphmw_comm_step(sphmw_ctx *c, const char *scheme, int nsteps) {
     SlabComm *m = c->comm;
-    const bool hopkins = !strcmp(scheme, "hopkins") || !strcmp(scheme, "hopkins_full");
-    if (!strcmp(scheme, "flow")) {
-        // isothermal_flow_witch.jl:221-232, operator by operator; inflow re-seeding and outflow by
-        // removal renumber particles across ranks: open box only
+    const bool hopkins = !strcmp(scheme, "hopkins") || !strcmp(scheme, "hopkins_full") || !strcmp(scheme, "hopkins_total");
+    const bool aflow = !strcmp(scheme, "aflow");
+    if (!strcmp(scheme, "flow") || aflow) {
+        // isothermal_flow_witch.jl:221-232 / adiabatic_flow_witch.jl:231-243, operator by operator;
+        // inflow re-seeding and outflow by removal renumber particles across ranks: open box only
         if (!m->open_box) {
-            sphmw_set_error("step: the flow scheme loses and gains particles; call sphmw_comm_open_box first");
+            sphmw_set_error("step: the %s scheme loses and gains particles; call sphmw_comm_open_box first", scheme);
             return SPHMW_E_STATE;
         }
         for (int k = 0; k < nsteps; ++k) {
             TRY(sphmw_apply_named(c, "flow.accelerate", 0));
-            TRY(sphmw_apply_named(c, "flow.move", 0));
-            TRY(comm_flow_spawn(c));
+            TRY(sphmw_apply_named(c, aflow ? "aflow.move" : "flow.move", 0));
+            TRY(comm_flow_spawn(c, aflow));
             TRY(comm_exchange_all(c));
             TRY(sphmw_build_cell_list(c, nullptr));
-            for (const char *op : {"flow.balance_of_mass", "flow.find_pressure", "flow.find_pot_temp", "flow.internal_force",
-                                   "flow.accelerate"})
-                TRY(sphmw_apply_named(c, op, 0));
+            if (aflow) {
+                TRY(sphmw_apply_named(c, "aflow.find_density", 1));  // self = true (:236)
+                for (const char *op : {"aflow.find_s", "aflow.find_pressure", "aflow.entropy_production",
+                                       "flow.internal_force", "flow.accelerate"})
+                    TRY(sphmw_apply_named(c, op, 0));
+            } else {
+                for (const char *op : {"flow.balance_of_mass", "flow.find_pressure", "flow.find_pot_temp",
+                                       "flow.internal_force", "flow.accelerate"})
+                    TRY(sphmw_apply_named(c, op, 0));
+            }
         }
         return SPHMW_OK;
     }
     if (strcmp(scheme, "wcsph") && !hopkins) {
-        sphmw_set_error("step: the fused 'wcsph', 'hopkins', 'hopkins_full' and the 'flow' schemes run on slabs");
+        sphmw_set_error("step: the fused 'wcsph', 'hopkins', 'hopkins_full', 'hopkins_total' and the 'flow' and "
+                        "'aflow' schemes run on slabs");
         return SPHMW_E_UNSUPPORTED_OP;
     }
     if (nsteps <= 0) return SPHMW_OK;
-    if (hopkins) {  // three pair passes per step, three ghost columns, plain schedule
+    if (hopkins) {  // three ghost columns, plain schedule (hopkins_total: operator by operator)
         for (int k = 0; k < nsteps; ++k) {
             TRY(sphmw_step_scheme_phase(c, scheme, 0));
             TRY(comm_exchange_all(c));

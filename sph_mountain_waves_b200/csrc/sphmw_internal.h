@@ -165,7 +165,7 @@ __device__ __forceinline__ bool neighbour_pkey(const Grid &g, const CellCoord &c
 #define TAG_OWNED 0u
 #define TAG_GHOST 1u
 #define TAG_DEAD 2u
-#define HALO_RECORD 13  // x0 x1 x2 v0 v1 v2 m h rho rho_p type idx kind
+#define HALO_RECORD 13  // the base record: x0 x1 x2 v0 v1 v2 m h rho rho_p type idx kind (halo_record.cuh)
 #define HALO_KIND_MIGRANT 0.0
 #define HALO_KIND_GHOST 1.0
 #define SLAB_LOST_CAP 4096u  // particles one rank may lose to the global box in one step (open box, slab_comm.cu)
@@ -353,6 +353,7 @@ struct sphmw_ctx {
     int64_t slab_check_want[4][2] = {};           // the host's figures for the same builds
     uint64_t slab_checks = 0;
     struct SlabComm *comm = nullptr;              // NCCL halo transport (slab_comm.cu)
+    int halo_kind = -1;                           // halo record kind (halo_record.cuh), fixed at first use; -1: not yet
     uint32_t *lost_list = nullptr;                // open box: [0] count, [1..] global indices the last pack dropped
     struct FrameAsync *frame_async = nullptr;     // asynchronous frame output / upload prefetch (frame_async.cu)
     uint32_t *halo_counters = nullptr;            // device: [0] left records [1] right records
@@ -477,8 +478,8 @@ int sphmw_materialize(sphmw_ctx *c, int slot);
 int64_t sphmw_list_ops(char *buf, int64_t cap);
 int sphmw_dump_pairs(sphmw_ctx *c, int64_t *pi, int64_t *pj, int64_t cap, int64_t *n);
 int sphmw_flow_add_particles(sphmw_ctx *c, int64_t *n_added, bool adiabatic);
-int sphmw_flow_collect_slab(sphmw_ctx *c, uint32_t *list, uint32_t *pos, uint32_t cap);  // slab contexts (slab_comm.cu)
-int sphmw_flow_spawn_slab(sphmw_ctx *c, const uint32_t *pos, const uint32_t *new_idx, int m);
+int sphmw_flow_collect_slab(sphmw_ctx *c, uint32_t *list, uint32_t *pos, uint32_t cap, bool adiabatic);  // slab contexts (slab_comm.cu)
+int sphmw_flow_spawn_slab(sphmw_ctx *c, const uint32_t *pos, const uint32_t *new_idx, int m, bool adiabatic);
 int sphmw_pair_list_stats(sphmw_ctx *c, int64_t out[4]);
 int sphmw_tile_stats(sphmw_ctx *c, int64_t out[6]);
 int sphmw_ensure_records(sphmw_ctx *c);  // api.cu: allocate the packed neighbour records
@@ -495,6 +496,8 @@ int sphmw_exclusive_scan_u32(sphmw_ctx *c, uint32_t *data, int64_t n);
 // implemented in halo.cu / slab_comm.cu
 int sphmw_halo_pack_enqueue(sphmw_ctx *c, double *msg_left, double *msg_right, int64_t cap_records, bool edge_only);
 int sphmw_halo_pack_collect_nowait(sphmw_ctx *c, int64_t cap_records, int64_t counts[5]);
+int sphmw_halo_kind(sphmw_ctx *c, int *kind);  // HALO_REC_BASE / HALO_REC_ADIABATIC (halo_record.cuh)
+int sphmw_comm_add_new_particles(sphmw_ctx *c, int64_t *n_added, bool adiabatic);
 int sphmw_comm_step(sphmw_ctx *c, const char *scheme, int nsteps);
 int sphmw_comm_create_cell_list(sphmw_ctx *c, int64_t *n_alive);
 void sphmw_comm_free(sphmw_ctx *c);

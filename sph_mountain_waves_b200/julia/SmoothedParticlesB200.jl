@@ -74,7 +74,9 @@ Same contract as structs.jl:43-92: particles of type `T`, removed once outside t
 (SPHMW_FLAG_*), and for x-slabs over several GPUs `rank`, `world`, `nccl_id` (128 bytes from
 `comm_unique_id()`, the same on every rank), `halo_capacity`, `open_box` (particles may leave the
 bounding box: the library then replays the swap-from-end renumbering of core.jl:72-81 across ranks
-after every halo exchange, `sphmw_comm_open_box`).
+after every halo exchange, `sphmw_comm_open_box`).  The adiabatic flow driver ("aflow") runs on slabs
+with `open_box=true`; hopkins_total needs `flags=SPHMW_FLAG_GHOST3` (three ghost columns), like the
+other Hopkins drivers.
 """
 mutable struct ParticleSystem{T<:AbstractParticle}
     h::Float64
@@ -315,7 +317,9 @@ end
 ≙ add_new_particles!(sys) of the constant-U flow drivers (isothermal_flow_witch.jl:175-186 under scheme
 "flow", adiabatic_flow_witch.jl:197-208 under "aflow"): INFLOW particles that entered the domain turn
 FLUID and a successor is created bc_width upstream with the driver's Particle constructor — on the
-device.  Returns the number of particles added.
+device.  Returns the number of particles added.  On x-slabs (`open_box=true`) the call is collective:
+every rank makes the successors of its own particles with the reference's global indices, and the
+number returned is the total over all ranks, as on one GPU.
 """
 function add_new_particles!(sys::ParticleSystem)
     before_device_call!(sys)

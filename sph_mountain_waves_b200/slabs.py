@@ -32,7 +32,7 @@ from .schemes import wcsph_perturbed_witch as wpw
 
 GHOST_COLS = 2
 GHOST3_FLAG = 256  # SPHMW_FLAG_GHOST3: three ghost columns per side (the Hopkins schemes)
-RECORD = 13  # x0 x1 x2 v0 v1 v2 m h rho rho_p type idx kind
+RECORD = 13  # the base record: x0 x1 x2 v0 v1 v2 m h rho rho_p type idx kind (csrc/halo_record.cuh)
 KIND_MIGRANT, KIND_GHOST = 0.0, 1.0
 
 
@@ -121,7 +121,7 @@ def global_indices(group_counts_all: np.ndarray, rank: int) -> np.ndarray:
 
 # ----------------------------------------------------------------------------- transport
 def exchange(plan: SlabPlan, send_left, send_right, migr_left: int, migr_right: int, empty: Callable):
-    """Move halo records to the x-adjacent ranks.  `send_*` are (count, RECORD) float64
+    """Move halo records to the x-adjacent ranks.  `send_*` are (count, width) float64
     tensors (or None when there is no neighbour); `empty(n)` allocates a receive tensor on
     the right device.  Returns ((recv_from_left, n_migrants), (recv_from_right, n_migrants))."""
     import torch
@@ -168,21 +168,41 @@ class LibSlabBackend:
         import torch
         self.sys, self.plan = sys, plan
         self.cap = int(cap_records)
-        dev = torch.device("cuda", sys.device)
-        self.buf_l = torch.empty((self.cap, RECORD), dtype=torch.float64, device=dev) if plan.has_left else None
-        self.buf_r = torch.empty((self.cap, RECORD), dtype=torch.float64, device=dev) if plan.has_right else None
-        self.dev = dev
+        self.dev = torch.device("cuda", sys.device)
+        self._width = None
+        self.buf_l = self.buf_r = None
         self.lost = 0
+
+    @property
+    def width(self) -> int:
+        """doubles per record: RECORD, or more for a context that carries extra state (the adiabatic flow
+        driver's S, P, T, theta).  Asked when first needed — after the particles are on the device — and
+        fixed by the library from then on."""
+        if self._width is None:
+            self.sys._flush()
+            w = C.c_int32()
+            check(_capi.lib().sphmw_halo_record_width(self.sys.ctx, C.byref(w)))
+            self._width = w.value
+        return self._width
+
+    def _buffers(self):
+        import torch
+        if self.buf_l is None and self.buf_r is None:
+            shape = (self.cap, self.width)
+            self.buf_l = torch.empty(shape, dtype=torch.float64, device=self.dev) if self.plan.has_left else None
+            self.buf_r = torch.empty(shape, dtype=torch.float64, device=self.dev) if self.plan.has_right else None
 
     def empty(self, n: int):
         import torch
-        return torch.empty((n, RECORD), dtype=torch.float64, device=self.dev)
+        return torch.empty((n, self.width), dtype=torch.float64, device=self.dev)
 
     @property
     def scheme(self) -> bytes:
-        """the fused scheme this context steps: "wcsph", or "hopkins"/"hopkins_full" (three ghost columns)"""
+        """the scheme this context steps: "wcsph", "hopkins"/"hopkins_full"/"hopkins_total" (three ghost
+        columns) or "aflow" (the adiabatic flow driver; a step in which an INFLOW particle converts needs the
+        library transport with the open box)"""
         s = getattr(self.sys.T, "scheme", "wcsph")
-        return s.encode() if s in ("hopkins", "hopkins_full") else b"wcsph"
+        return s.encode() if s in ("hopkins", "hopkins_full", "hopkins_total", "aflow") else b"wcsph"
 
     def pre(self):
         check(_capi.lib().sphmw_step_phase(self.sys.ctx, self.scheme, 0))
@@ -194,6 +214,7 @@ class LibSlabBackend:
         self.sys.create_cell_list(want_count=False)
 
     def pack(self):
+        self._buffers()
         counts = (C.c_int64 * 5)()
         pl = C.c_void_p(self.buf_l.data_ptr()) if self.buf_l is not None else None
         pr = C.c_void_p(self.buf_r.data_ptr()) if self.buf_r is not None else None
@@ -219,6 +240,7 @@ class LibSlabBackend:
         """finish the current step and start the next one: edge columns first (force, kick,
         drift, pack), then the interior — everything is only enqueued"""
         lib = _capi.lib()
+        self._buffers()
         check(lib.sphmw_step_phase(self.sys.ctx, b"wcsph", 2))
         pl = C.c_void_p(self.buf_l.data_ptr()) if self.buf_l is not None else None
         pr = C.c_void_p(self.buf_r.data_ptr()) if self.buf_r is not None else None
@@ -369,7 +391,7 @@ class SlabRun:
         """Slice a whole (small) case held on the host: reference indices are the positions in
         `case.fields`.  Used by tests and by single-process multi-context runs.  A Hopkins case gets
         three ghost columns per side (SPHMW_FLAG_GHOST3)."""
-        ghost = 3 if case.scheme in ("hopkins", "hopkins_full") else GHOST_COLS
+        ghost = 3 if case.scheme in ("hopkins", "hopkins_full", "hopkins_total") else GHOST_COLS
         if ghost == 3:
             flags |= GHOST3_FLAG
         plan = plan_slab(case.box_min, case.box_max, case.h, rank, world, ghost=ghost)
