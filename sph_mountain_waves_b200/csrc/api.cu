@@ -334,6 +334,7 @@ extern "C" int sphmw_destroy(sphmw_ctx *c) {
     cudaFree(c->cell_start); cudaFree(c->scan_tmp); cudaFree(c->removed);
     cudaFree(c->mv_old); cudaFree(c->mv_new);
     cudaFree(c->d_counters); cudaFree(c->staging); cudaFree(c->reduce_tmp);
+    cudaFree(c->fluid_flag); cudaFree(c->fluid_work); cudaFree(c->fluid_tiles);
     cudaFree(c->xq); cudaFree(c->pl.list); cudaFree(c->pl.list16); cudaFree(c->pl.cnt); cudaFree(c->tile_tab);
     for (int k = 0; k < 3; ++k) cudaFree(c->rec[k]);
     if (c->h_removed) cudaFreeHost(c->h_removed);
@@ -448,6 +449,7 @@ extern "C" int sphmw_resize(sphmw_ctx *c, int64_t n) {
     c->n = n;
     c->n_owned = n;
     c->cell_list_valid = false;
+    c->keys_from_advance = false;
     return SPHMW_OK;
 }
 extern "C" int sphmw_count(sphmw_ctx *c, int64_t *n) {
@@ -515,8 +517,9 @@ extern "C" int sphmw_upload(sphmw_ctx *c, const char *field, const double *buf, 
                                                               c->staging + (int64_t)k * n, c->idx, n);
         c->stale[slot] = false;
     }
-    if (d->slot == S_X0) c->cell_list_valid = false;
+    if (d->slot == S_X0) c->cell_list_valid = false, c->keys_from_advance = false;
     if (d->slot == S_DV0) c->dv_zero = false;
+    if (d->slot == S_TYPE) c->fluid_gen = ~0ull;  // the fluid work list no longer matches the types
     CUDA_TRY(cudaGetLastError());
     // staging is reused by the next call: the copy out of `buf` must be complete
     // before we return anyway (host memory is only borrowed).

@@ -20,6 +20,11 @@ struct GatherList {
     // packed neighbour record A {x, y, z, m} (SPHMW_FLAG_PACKED_RECORDS; null otherwise)
     int mpos;
     NbRec *recA;
+    // fluid flag per position (type == fluid, the test of wcsph_force_finish), the input of the fluid
+    // work list (cell_list.cu); null: not wanted
+    int tpos;  // entry of the type field in the lists above
+    double fluid;
+    uint8_t *fl;
 };
 
 __global__ void k_gather(GatherList gl, const uint32_t *__restrict__ src,
@@ -43,6 +48,7 @@ __global__ void k_gather(GatherList gl, const uint32_t *__restrict__ src,
         const double v = gl.from[f][s];
         gl.to[f][slot] = v;
         if (f == gl.mpos) ra[3] = v;
+        if (f == gl.tpos && gl.fl) gl.fl[slot] = v == gl.fluid;
 #pragma unroll
         for (int a = 0; a < 3; ++a)
             if (f == gl.xpos[a]) {

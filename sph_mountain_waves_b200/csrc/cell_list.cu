@@ -70,27 +70,7 @@ __global__ void k_keys(const double *__restrict__ x0, const double *__restrict__
         return;
     }
     if (pos >= n) return;
-    double x = x0[pos], y = x1[pos], z = DIM == 3 ? x2[pos] : 0.0;
-    // geometry.jl:24-30 — closed intervals; NaN fails every comparison
-    bool inside = g.box[0] <= x && x <= g.box[3] && g.box[1] <= y && y <= g.box[4] &&
-                  g.box[2] <= z && z <= g.box[5];
-    uint32_t k, ci = 0;
-    if (inside) {
-        // structs.jl:99-102 — IEEE division, then floor (never a reciprocal multiply)
-        long long i = (long long)floor(x / g.h) - g.phase[0];
-        long long j = (long long)floor(y / g.h) - g.phase[1];
-        long long kk = DIM == 3 ? (long long)floor(z / g.h) - g.phase[2] : 0;
-        // structs.jl:102 gives the reference key i + Lx*(j + Ly*k); stored is its physical image
-        k = pkey_ijk(g, (int)i, (int)j, (int)kk);
-        ci = (uint32_t)i;
-    }
-    if (!inside) {
-        k = (uint32_t)g.pkey_max;  // dead bucket: sorted behind every live cell
-        uint32_t slot = atomicAdd(&removed[0], 1u);
-        if (slot < removed_cap) removed[1 + slot] = idx[pos];
-    }
-    key[pos] = k;
-    cellx[pos] = ci;
+    cell_key_whole<DIM>(g, x0[pos], x1[pos], DIM == 3 ? x2[pos] : 0.0, pos, key, cellx, removed, removed_cap, idx);
 }
 
 // ---------------------------------------------------------------------------
@@ -204,6 +184,108 @@ int sphmw_exclusive_scan_u32(sphmw_ctx *c, uint32_t *data, int64_t n) {
 }
 
 // ---------------------------------------------------------------------------
+// fluid work list (pair_list.cuh k_binary_list_fluid): a stable compaction of the gather's fluid
+// flags — per-tile counts, an exclusive scan of them, then every position to its slot: a fluid one
+// after the fluid positions before it, any other after all fluid ones and the others before it
+// ---------------------------------------------------------------------------
+#define FL_ITEMS 8
+#define FL_TILE (256 * FL_ITEMS)
+
+__device__ __forceinline__ unsigned fl_load(const uint8_t *__restrict__ fl, int64_t base, int64_t n, uint8_t v[FL_ITEMS]) {
+    unsigned cnt = 0;
+    if (base + FL_ITEMS <= n) {
+        const uint2 w = *(const uint2 *)(fl + base);  // base is a multiple of 8
+#pragma unroll
+        for (int i = 0; i < FL_ITEMS; ++i) v[i] = (uint8_t)((i < 4 ? w.x >> (8 * i) : w.y >> (8 * (i - 4))) & 1u);
+    } else {
+#pragma unroll
+        for (int i = 0; i < FL_ITEMS; ++i) v[i] = base + i < n ? fl[base + i] : 0;
+    }
+#pragma unroll
+    for (int i = 0; i < FL_ITEMS; ++i) cnt += v[i];
+    return cnt;
+}
+
+__global__ void __launch_bounds__(256) k_fluid_count(const uint8_t *__restrict__ fl, int64_t n, uint32_t *__restrict__ tiles) {
+    __shared__ unsigned ws[8];
+    uint8_t v[FL_ITEMS];
+    unsigned cnt = fl_load(fl, blockIdx.x * (int64_t)FL_TILE + threadIdx.x * FL_ITEMS, n, v);
+    cnt = __reduce_add_sync(0xffffffffu, cnt);
+    if ((threadIdx.x & 31) == 0) ws[threadIdx.x >> 5] = cnt;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        unsigned t = 0;
+        for (int w = 0; w < 8; ++w) t += ws[w];
+        tiles[blockIdx.x] = t;
+    }
+}
+
+// the tile's positions are ordered in shared memory (fluid ones first) and written out as two
+// contiguous runs: a thread writing its own eight slots would scatter each warp store over 32 sectors
+__global__ void __launch_bounds__(256) k_fluid_scatter(const uint8_t *__restrict__ fl, int64_t n,
+                                                       const uint32_t *__restrict__ tiles, int64_t ntiles,
+                                                       uint32_t *__restrict__ work) {
+    __shared__ unsigned ws[8];
+    __shared__ uint32_t stage[FL_TILE];
+    const int64_t tile0 = blockIdx.x * (int64_t)FL_TILE;
+    const unsigned first = threadIdx.x * FL_ITEMS;
+    uint8_t v[FL_ITEMS];
+    const unsigned cnt = fl_load(fl, tile0 + first, n, v);
+    const unsigned lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    unsigned incl = cnt;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const unsigned t = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= (unsigned)o) incl += t;
+    }
+    if (lane == 31) ws[w] = incl;
+    __syncthreads();
+    unsigned fb = incl - cnt, ftile = 0;  // fluid positions of the tile before `first`, and in all
+    for (unsigned k = 0; k < 8; ++k) {
+        if (k < w) fb += ws[k];
+        ftile += ws[k];
+    }
+    const unsigned len = (unsigned)(n - tile0 < FL_TILE ? n - tile0 : FL_TILE);
+#pragma unroll
+    for (int i = 0; i < FL_ITEMS; ++i) {
+        const unsigned l = first + i;
+        if (l >= len) break;
+        if (v[i]) stage[fb++] = (uint32_t)(tile0 + l);
+        else stage[ftile + l - fb] = (uint32_t)(tile0 + l);
+    }
+    __syncthreads();
+    const uint32_t fbase = tiles[blockIdx.x];  // fluid positions before the tile
+    const uint32_t obase = tiles[ntiles] + (uint32_t)tile0 - fbase;  // all fluid ones + the others before it
+    for (unsigned l = threadIdx.x; l < len; l += 256)
+        work[l < ftile ? fbase + l : obase + (l - ftile)] = stage[l];
+}
+
+static int build_fluid_list(sphmw_ctx *c, int64_t n) {
+    const int64_t ntiles = (n + FL_TILE - 1) / FL_TILE;
+    if (ntiles + 1 > c->fluid_tiles_cap) {
+        cudaFree(c->fluid_tiles);
+        c->fluid_tiles = nullptr;
+        c->fluid_tiles_cap = (c->cap + FL_TILE - 1) / FL_TILE + 1;
+        CUDA_TRY(cudaMalloc(&c->fluid_tiles, sizeof(uint32_t) * c->fluid_tiles_cap));
+    }
+    {
+        TIMED(c, "fluid_list");
+        k_fluid_count<<<(unsigned)ntiles, 256, 0, c->stream>>>(c->fluid_flag, n, c->fluid_tiles);
+    }
+    CUDA_TRY(cudaMemsetAsync(c->fluid_tiles + ntiles, 0, sizeof(uint32_t), c->stream));
+    TRY(sphmw_exclusive_scan_u32(c, c->fluid_tiles, ntiles + 1));
+    {
+        TIMED(c, "fluid_list");
+        k_fluid_scatter<<<(unsigned)ntiles, 256, 0, c->stream>>>(c->fluid_flag, n, c->fluid_tiles, ntiles, c->fluid_work);
+    }
+    CUDA_TRY(cudaGetLastError());
+    c->fluid_count = c->fluid_tiles + ntiles;
+    c->fluid_gen = c->cell_gen;
+    c->fluid_value = c->prm.fluid;
+    return SPHMW_OK;
+}
+
+// ---------------------------------------------------------------------------
 // scatter, in-cell ordering, gather
 // ---------------------------------------------------------------------------
 __global__ void k_scatter(const uint32_t *__restrict__ key, const uint32_t *__restrict__ rank,
@@ -306,6 +388,7 @@ int sphmw_build_cell_list(sphmw_ctx *c, int64_t *n_alive) {
         TRY(sphmw_publish_words(c, (const uint32_t *)(c->d_counters + 2), (uint32_t *)(c->h_counters + 2), 2, c->stream));
     }
     if (n == 0) {
+        c->keys_from_advance = false;
         CUDA_TRY(cudaMemsetAsync(c->cell_start, 0, sizeof(uint32_t) * (ncells + 2), c->stream));
         c->cell_list_valid = true;
         c->n_owned = 0;
@@ -323,8 +406,11 @@ int sphmw_build_cell_list(sphmw_ctx *c, int64_t *n_alive) {
         CUDA_TRY(cudaMalloc(&c->scan_tmp, sizeof(uint32_t) * c->scan_tmp_len));
     }
 
-    CUDA_TRY(cudaMemsetAsync(c->removed, 0, sizeof(uint32_t) * 2, c->stream));
-    {
+    // keys written by the force pass's advance (pair_ops.cu run_fused_force): same function, same x
+    const bool keyed = c->keys_from_advance && c->slab_lo < 0;
+    c->keys_from_advance = false;
+    if (!keyed) {
+        CUDA_TRY(cudaMemsetAsync(c->removed, 0, sizeof(uint32_t) * 2, c->stream));
         TIMED(c, "cell_keys");
         const bool slab = c->slab_lo >= 0;
         const unsigned gr = grid_for(n, 256);
@@ -450,6 +536,16 @@ int sphmw_build_cell_list(sphmw_ctx *c, int64_t *n_alive) {
     for (int a = 0; a < 3; ++a) gl.xpos[a] = -1;
     gl.mpos = -1;
     gl.recA = nullptr;
+    gl.tpos = -1;
+    gl.fluid = c->prm.fluid;
+    gl.fl = nullptr;
+    c->fluid_gen = ~0ull;
+    const bool fluid_list = c->want_fluid_list && c->allocated[S_TYPE] && !c->stale[S_TYPE] && n_new > 0;
+    if (fluid_list && !c->fluid_work) {
+        CUDA_TRY(cudaMalloc(&c->fluid_flag, (size_t)c->cap + 8));
+        CUDA_TRY(cudaMalloc(&c->fluid_work, sizeof(uint32_t) * (size_t)c->cap));
+    }
+    if (fluid_list) gl.fl = c->fluid_flag;
     if (sphmw_use_records(c) && c->allocated[S_M] && !c->stale[S_M]) {
         TRY(sphmw_ensure_records(c));
         gl.recA = c->rec[0];
@@ -462,6 +558,7 @@ int sphmw_build_cell_list(sphmw_ctx *c, int64_t *n_alive) {
             gathered[gl.count] = s;
             if (s >= S_X0 && s <= S_X2) gl.xpos[s - S_X0] = gl.count;
             if (s == S_M) gl.mpos = gl.count;
+            if (s == S_TYPE) gl.tpos = gl.count;
             ++gl.count;
         }
     if (n_new > 0) {
@@ -472,6 +569,7 @@ int sphmw_build_cell_list(sphmw_ctx *c, int64_t *n_alive) {
     }
     c->pos_valid = false;  // rebuilt on demand (sphmw_ensure_pos_of_idx)
     CUDA_TRY(cudaGetLastError());
+    if (fluid_list) TRY(build_fluid_list(c, n_new));
     for (int f = 0; f < gl.count; ++f) std::swap(c->cur.s[gathered[f]], c->alt.s[gathered[f]]);
     std::swap(c->idx, c->idx_alt);
     std::swap(c->key, c->rank);

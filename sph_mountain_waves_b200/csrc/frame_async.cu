@@ -333,8 +333,9 @@ extern "C" int sphmw_upload_commit(sphmw_ctx *c) {
                 k_permute_in_async<<<grid_for(n, 256), 256, 0, c->stream>>>(c->cur.s[slot], fa->up_dev + it.off + (size_t)k * n, n);
             }
             c->stale[slot] = false;
-            if (slot == S_X0) c->cell_list_valid = false;
+            if (slot == S_X0) c->cell_list_valid = false, c->keys_from_advance = false;
             if (slot == S_DV0) c->dv_zero = false;
+            if (slot == S_TYPE) c->fluid_gen = ~0ull;
         }
     CUDA_TRY(cudaGetLastError());
     CUDA_TRY(cudaEventRecord(fa->up_consumed, c->stream));

@@ -313,6 +313,7 @@ k_binary_build(Fields f, Fields out, Params prm, Grid g, const uint32_t *__restr
     }
     if (self) op.template pair<DIM>(f, prm, p, p, 0.0, 0.0, 0.0, 0.0);  // core.jl:155-157
     op.template finish<DIM>(f, out, prm, p);
+    op.template after<DIM>(g, out, prm, p);
     if constexpr (REC && Op::REC_KIND == 1) {
         // what finish() just stored for p (same thread: reads see its own writes), as records
         nb_store(pl.recB + p, f.s[S_V0][p], f.s[S_V1][p], DIM == 3 ? f.s[S_V2][p] : 0.0, f.s[S_H][p]);
@@ -323,14 +324,17 @@ k_binary_build(Fields f, Fields out, Params prm, Grid g, const uint32_t *__restr
     nl_count_pairs(pair_counter, accepted);
 }
 
-// REC (fused force pass only): entries are evaluated from the packed records
+// REC (fused force pass only): entries are evaluated from the packed records.
+// pairs == false (a non-fluid particle of an Op with PAIRS_FOR_FLUID_ONLY): the recorded entries are
+// not evaluated — finish() would discard their sums — but still counted, so the pair counter keeps the
+// reference's figure; a particle without a list (NL_NONE) walks the cells as always.
 template <int DIM, class Op, bool REC>
 __device__ __forceinline__ void nl_list_particle(int64_t p, const Fields &f, const Fields &out, const Params &prm,
                                                  const Grid &g, const uint32_t *__restrict__ key,
                                                  const uint32_t *__restrict__ cellx,
                                                  const uint32_t *__restrict__ cell_start, int self,
                                                  unsigned long long *pair_counter, const ColFilter &cf,
-                                                 const PairList &pl) {
+                                                 const PairList &pl, bool pairs = true) {
     const CellCoord home = cell_of(g, key[p], cellx[p]);
     if (cf.on && !col_selected(cf, home.i)) {
         if (cf.copy) Op::template skip<DIM>(f, out, p);
@@ -341,7 +345,9 @@ __device__ __forceinline__ void nl_list_particle(int64_t p, const Fields &f, con
     Op op;
     op.template init<DIM>(f, prm, p);
     unsigned accepted = 0;
-    if (cnt != NL_NONE) {
+    if (cnt != NL_NONE && !pairs) {
+        accepted = cnt;  // the recording pass accepted exactly these entries (same positions)
+    } else if (cnt != NL_NONE) {
         const uint32_t *row = pl.list + ((size_t)(p >> 5) * (uint32_t)pl.stride) * 32 + (size_t)(p & 31);
         // (loading the next entry's position one iteration ahead as well was measured slower:
         // profiles/r01b_pair_list.md)
@@ -358,6 +364,7 @@ __device__ __forceinline__ void nl_list_particle(int64_t p, const Fields &f, con
     }
     if (self) op.template pair<DIM>(f, prm, p, p, 0.0, 0.0, 0.0, 0.0);
     op.template finish<DIM>(f, out, prm, p);
+    op.template after<DIM>(g, out, prm, p);
     nl_count_pairs(pair_counter, accepted);
 }
 
@@ -374,6 +381,25 @@ k_binary_list(Fields f, Fields out, Params prm, Grid g, const uint32_t *__restri
     const int64_t p = blockIdx.x * (int64_t)NL_BLOCK + threadIdx.x;
     if (p >= n) return;
     nl_list_particle<DIM, Op, REC>(p, f, out, prm, g, key, cellx, cell_start, self, pair_counter, cf, pl);
+}
+
+// Replaying pass of an Op with PAIRS_FOR_FLUID_ONLY over the fluid work list of this cell-list
+// generation (cell_list.cu k_fluid_scatter): work[0, *n_fluid) are the fluid positions ascending, the
+// rest the other positions ascending.  Thread t handles p = work[t]; the list row of p and the order of
+// its sum are those of k_binary_list, so every bit is too.  Whole warps run the pair loop or skip it
+// (only the warp that straddles *n_fluid diverges), where a per-thread test would leave every warp
+// that holds a fluid particle running the loop for all its lanes.
+template <int DIM, class Op, bool REC = false>
+__global__ void NL_LIST_BOUNDS
+k_binary_list_fluid(Fields f, Fields out, Params prm, Grid g, const uint32_t *__restrict__ key,
+                    const uint32_t *__restrict__ cellx, const uint32_t *__restrict__ cell_start, int64_t n,
+                    int self, unsigned long long *pair_counter, ColFilter cf, PairList pl,
+                    const uint32_t *__restrict__ work, const uint32_t *__restrict__ n_fluid) {
+    static_assert(Op::PAIRS_FOR_FLUID_ONLY, "k_binary_list_fluid skips the pairs of non-fluid particles");
+    const int64_t t = blockIdx.x * (int64_t)NL_BLOCK + threadIdx.x;
+    if (t >= n) return;
+    nl_list_particle<DIM, Op, REC>((int64_t)work[t], f, out, prm, g, key, cellx, cell_start, self, pair_counter, cf, pl,
+                                   t < (int64_t)*n_fluid);
 }
 
 // The particles of the cell columns [a0, a1] and [b0, b1] are two contiguous ranges of the zrun
@@ -411,6 +437,8 @@ k_binary_list_cols(Fields f, Fields out, Params prm, Grid g, const uint32_t *__r
     const uint32_t total = r.n0 + r.n1;
     for (uint32_t t = blockIdx.x * NL_BLOCK + threadIdx.x; t < total; t += gridDim.x * NL_BLOCK) {
         const int64_t p = t < r.n0 ? (int64_t)r.b0 + t : (int64_t)r.b1 + (t - r.n0);
-        if (p < n) nl_list_particle<DIM, Op, REC>(p, f, out, prm, g, key, cellx, cell_start, self, pair_counter, cf, pl);
+        if (p < n)
+            nl_list_particle<DIM, Op, REC>(p, f, out, prm, g, key, cellx, cell_start, self, pair_counter, cf, pl,
+                                           !Op::PAIRS_FOR_FLUID_ONLY || f.s[S_TYPE][p] == prm.fluid);
     }
 }

@@ -81,6 +81,7 @@ k_binary(Fields f, Fields out, Params prm, Grid g, const uint32_t *__restrict__ 
     }
     if (self) op.template pair<DIM>(f, prm, p, p, 0.0, 0.0, 0.0, 0.0);  // core.jl:155-157
     op.template finish<DIM>(f, out, prm, p);
+    op.template after<DIM>(g, out, prm, p);
     if (pair_counter) {
         unsigned m = __activemask();
         unsigned tot = __reduce_add_sync(m, (unsigned)cnt);
@@ -238,6 +239,7 @@ static int need_slots(sphmw_ctx *c, const SlotList &reads, const SlotList &write
 
 template <class Op>
 static int run_unary(sphmw_ctx *c, const char *name) {
+    c->keys_from_advance = false;  // the operator may move particles
     if (c->n == 0) return SPHMW_OK;
     TIMED(c, name);
     if (c->grid.dim == 2)
@@ -347,11 +349,22 @@ static int run_binary_cols(sphmw_ctx *c, const char *name, int self, const Field
         // their particle ranges, which are contiguous in the zrun cell order
         const bool cols = cf.on && cf.sparse && !cf.copy && c->grid.zrun && !getenv("SPHMW_NO_COLUMN_RANGES");
         const unsigned cblocks = std::min<unsigned>(blocks, (unsigned)c->sm_count * 8u);
+        // an Op whose finish() discards the pair sums of non-fluid particles runs over the fluid work
+        // list of this cell list: the pair loop for the fluid positions only (pair_list.cuh)
+        bool fluid = false;
+        if constexpr (Op::PAIRS_FOR_FLUID_ONLY)
+            fluid = !cols && c->fluid_gen == c->cell_gen && c->fluid_value == c->prm.fluid;
+#define NL_FLUID_ARGS NL_ARGS, c->pl, c->fluid_work, c->fluid_count
         if constexpr (REC) {
             if (rec && c->rec_bc_gen == c->cell_gen) {
                 if (cols) {
                     if (c->grid.dim == 2) k_binary_list_cols<2, Op, true><<<cblocks, NL_BLOCK, 0, c->stream>>>(NL_ARGS, c->pl);
                     else k_binary_list_cols<3, Op, true><<<cblocks, NL_BLOCK, 0, c->stream>>>(NL_ARGS, c->pl);
+                } else if (fluid) {
+                    if constexpr (Op::PAIRS_FOR_FLUID_ONLY) {
+                        if (c->grid.dim == 2) k_binary_list_fluid<2, Op, true><<<blocks, NL_BLOCK, 0, c->stream>>>(NL_FLUID_ARGS);
+                        else k_binary_list_fluid<3, Op, true><<<blocks, NL_BLOCK, 0, c->stream>>>(NL_FLUID_ARGS);
+                    }
                 } else {
                     if (c->grid.dim == 2) k_binary_list<2, Op, true><<<blocks, NL_BLOCK, 0, c->stream>>>(NL_ARGS, c->pl);
                     else k_binary_list<3, Op, true><<<blocks, NL_BLOCK, 0, c->stream>>>(NL_ARGS, c->pl);
@@ -363,6 +376,11 @@ static int run_binary_cols(sphmw_ctx *c, const char *name, int self, const Field
         if (cols) {
             if (c->grid.dim == 2) k_binary_list_cols<2, Op><<<cblocks, NL_BLOCK, 0, c->stream>>>(NL_ARGS, c->pl);
             else k_binary_list_cols<3, Op><<<cblocks, NL_BLOCK, 0, c->stream>>>(NL_ARGS, c->pl);
+        } else if (fluid) {
+            if constexpr (Op::PAIRS_FOR_FLUID_ONLY) {
+                if (c->grid.dim == 2) k_binary_list_fluid<2, Op><<<blocks, NL_BLOCK, 0, c->stream>>>(NL_FLUID_ARGS);
+                else k_binary_list_fluid<3, Op><<<blocks, NL_BLOCK, 0, c->stream>>>(NL_FLUID_ARGS);
+            }
         } else if (c->grid.dim == 2)
             k_binary_list<2, Op><<<blocks, NL_BLOCK, 0, c->stream>>>(NL_ARGS, c->pl);
         else
@@ -406,6 +424,7 @@ static int run_binary_cols(sphmw_ctx *c, const char *name, int self, const Field
             k_binary<3, Op><<<blocks, 128, 0, c->stream>>>(NL_ARGS);
     }
 #undef NL_ARGS
+#undef NL_FLUID_ARGS
     CUDA_TRY(cudaGetLastError());
     return SPHMW_OK;
 }
@@ -626,6 +645,8 @@ int sphmw_apply_named(sphmw_ctx *c, const char *op, int self) {
                 // core.jl:151-161: `self` only matters for binary operators
                 self = 0;
             }
+            c->fluid_gen = ~0ull;  // an operator may change a particle's type (inflow conversion)
+            c->keys_from_advance = false;  // ... or its position
             return e->run(c, e->name, self);
         }
     sphmw_set_error("operator '%s' is not in the device menu (no CPU fallback)", op);
@@ -783,6 +804,7 @@ int sphmw_flow_spawn_slab(sphmw_ctx *c, const uint32_t *pos, const uint32_t *new
 #undef SPAWN_LIST
     CUDA_TRY(cudaGetLastError());
     c->n = n + m;
+    c->keys_from_advance = false;
     c->n_owned += m;
     c->cell_list_valid = false;
     return SPHMW_OK;
@@ -840,6 +862,7 @@ int sphmw_flow_add_particles(sphmw_ctx *c, int64_t *n_added, bool adiabatic) {
     }
     CUDA_TRY(cudaGetLastError());
     c->n = n + m;
+    c->keys_from_advance = false;
     c->n_owned = c->n;
     c->cell_list_valid = false;
     if (n_added) *n_added = m;
@@ -913,16 +936,34 @@ static int run_fused_density(sphmw_ctx *c) {
     return rec ? run_binary<B_wcsph_density_fused, true>(c, name, 0, c->cur, 1)
                : run_binary<B_wcsph_density_fused>(c, name, 0, c->cur, 1);
 }
+static int run_force_advance(sphmw_ctx *c, const char *name, const ColFilter &cf) {
+    const bool rec = sphmw_use_records(c);
+    if (c->flags & SPHMW_FLAG_FAST_MATH)
+        return rec ? run_binary_cols<B_force_advance<B_wcsph_momentum_fast>, true>(c, name, 0, c->alt, cf)
+                   : run_binary_cols<B_force_advance<B_wcsph_momentum_fast>>(c, name, 0, c->alt, cf);
+    return rec ? run_binary_cols<B_force_advance<B_wcsph_momentum_fused>, true>(c, name, 0, c->alt, cf)
+               : run_binary_cols<B_force_advance<B_wcsph_momentum_fused>>(c, name, 0, c->alt, cf);
+}
 static int run_fused_force(sphmw_ctx *c, const char *name, const ColFilter &cf, bool advance = false) {
     const bool rec = sphmw_use_records(c);
-    if (advance) {
-        // + the next step's accelerate! and move! in finish() (B_force_advance); x and v go to alt
-        if (c->flags & SPHMW_FLAG_FAST_MATH)
-            return rec ? run_binary_cols<B_force_advance<B_wcsph_momentum_fast>, true>(c, name, 0, c->alt, cf)
-                       : run_binary_cols<B_force_advance<B_wcsph_momentum_fast>>(c, name, 0, c->alt, cf);
-        return rec ? run_binary_cols<B_force_advance<B_wcsph_momentum_fused>, true>(c, name, 0, c->alt, cf)
-                   : run_binary_cols<B_force_advance<B_wcsph_momentum_fused>>(c, name, 0, c->alt, cf);
+    if (advance && c->slab_lo < 0 && c->n > 0) {
+        // + the next step's accelerate! and move! in finish() (B_force_advance); x and v go to alt.  The
+        // thread that drifts a particle also writes the next cell list's key of it, and the removed list
+        // of the next build starts here: that build then skips k_keys (cell_list.cu)
+        CUDA_TRY(cudaMemsetAsync(c->removed, 0, sizeof(uint32_t) * 2, c->stream));
+        c->prm.key_out = c->key;
+        c->prm.cellx_out = c->cellx;
+        c->prm.key_removed = c->removed;
+        c->prm.key_idx = c->idx;
+        c->prm.key_removed_cap = (uint32_t)c->removed_cap;
+        const int rc = run_force_advance(c, name, cf);
+        c->prm.key_out = c->prm.cellx_out = c->prm.key_removed = nullptr;
+        c->prm.key_idx = nullptr;
+        TRY(rc);
+        c->keys_from_advance = true;
+        return SPHMW_OK;
     }
+    if (advance) return run_force_advance(c, name, cf);  // slab: ghosts and migrants join after the drift
     if (tiles_enabled(c)) {
         if (c->flags & SPHMW_FLAG_FAST_MATH) return run_tiled<B_wcsph_momentum_fast>(c, name, 0, c->alt, cf);
         return run_tiled<B_wcsph_momentum_fused>(c, name, 0, c->alt, cf);
@@ -937,8 +978,15 @@ static int run_fused_force(sphmw_ctx *c, const char *name, const ColFilter &cf, 
 // slab mode: the halo exchange sits between the two halves (after the drift, before the sort)
 // advance: the force pass also opens the next step (accelerate! + move!, B_force_advance); the
 // context is then in the state step_wcsph_fused_pre leaves behind
+// the force pass of the fused step replays the pair list over the fluid work list (pair_list.cuh
+// k_binary_list_fluid): the cell-list builds from now on make one
+static void want_fluid_list(sphmw_ctx *c) {
+    c->want_fluid_list = !(c->flags & (SPHMW_FLAG_NO_PAIR_LIST | SPHMW_FLAG_CELL_PAIRS | SPHMW_FLAG_TILES));
+}
+
 static int step_wcsph_fused_post(sphmw_ctx *c, bool advance = false) {
     wcsph_before_sort(c);
+    want_fluid_list(c);
     TRY(sphmw_build_cell_list(c, nullptr));  // :313
     // :316-323
     for (int s : {S_RHO_BG, S_RHO_P, S_RHO, S_P_BG, S_P_P, S_P, S_PR2, S_CS}) {
@@ -1149,6 +1197,7 @@ static int step_wcsph_overlap_a(sphmw_ctx *c) {
     if (c->overlap_stage != 0) { sphmw_set_error("step_phase 2: an overlapped step is already in flight"); return SPHMW_E_STATE; }
     if (!c->dv_zero) { sphmw_set_error("step_phase 2: Dv must be zero (run step_phase 0 first)"); return SPHMW_E_STATE; }
     wcsph_before_sort(c);
+    want_fluid_list(c);
     TRY(sphmw_build_cell_list(c, nullptr));
     for (int s : {S_RHO_BG, S_RHO_P, S_RHO, S_P_BG, S_P_P, S_P, S_PR2, S_CS}) {
         TRY(sphmw_ensure_slot(c, s));
@@ -1295,6 +1344,7 @@ int sphmw_step_scheme_phase(sphmw_ctx *c, const char *scheme, int phase) {
 int sphmw_step_wcsph_phase(sphmw_ctx *c, int phase) { return sphmw_step_scheme_phase(c, "wcsph", phase); }
 
 int sphmw_step_scheme(sphmw_ctx *c, const char *scheme, int nsteps) {
+    c->keys_from_advance = false;  // only a step of this call may hand keys to the next build
     if (c->slab_lo >= 0 && nsteps > 0) {
         // with a communicator (sphmw_comm_init) the halo exchange is the library's business
         if (c->comm) return sphmw_comm_step(c, scheme, nsteps);

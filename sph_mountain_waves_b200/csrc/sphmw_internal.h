@@ -57,6 +57,11 @@ struct Params {
     double esc_h;
     long long esc_phase;
     int esc_lo, esc_hi;  // legal local columns after the drift: [esc_lo, esc_hi)
+    // whole-domain multi-step call: the force pass's advance also writes the next cell list's key of the
+    // new position (cell_key_whole, B_force_advance::after); null otherwise
+    uint32_t *key_out, *cellx_out, *key_removed;
+    const uint32_t *key_idx;
+    uint32_t key_removed_cap;
 };
 
 // neighbour-grid description passed to kernels by value (structs.jl:63-82)
@@ -157,6 +162,34 @@ __device__ __forceinline__ bool neighbour_pkey(const Grid &g, const CellCoord &c
     if (k < 0 || k >= (int)g.lim[2]) return false;  // <=> key + dkey outside 1..key_max
     pk = pkey_ijk(g, i, j, k);
     return true;
+}
+// find_key + is_inside of one particle of a whole-domain context (structs.jl:97-106, geometry.jl:24-30):
+// the physical key and column of position pos, or — outside the box (closed intervals; NaN fails every
+// comparison) — the dead bucket, with its reference index appended to the removed list.  Shared by the
+// cell-list build (k_keys) and the force pass's advance, so both compute the same bits.
+template <int DIM>
+__device__ __forceinline__ void cell_key_whole(const Grid &g, double x, double y, double z, int64_t pos,
+                                               uint32_t *__restrict__ key, uint32_t *__restrict__ cellx,
+                                               uint32_t *__restrict__ removed, uint32_t removed_cap,
+                                               const uint32_t *__restrict__ idx) {
+    const bool inside = g.box[0] <= x && x <= g.box[3] && g.box[1] <= y && y <= g.box[4] && g.box[2] <= z &&
+                        z <= g.box[5];
+    uint32_t k, ci = 0;
+    if (inside) {
+        // IEEE division, then floor (never a reciprocal multiply)
+        const long long i = (long long)floor(x / g.h) - g.phase[0];
+        const long long j = (long long)floor(y / g.h) - g.phase[1];
+        const long long kk = DIM == 3 ? (long long)floor(z / g.h) - g.phase[2] : 0;
+        // structs.jl:102 gives the reference key i + Lx*(j + Ly*k); stored is its physical image
+        k = pkey_ijk(g, (int)i, (int)j, (int)kk);
+        ci = (uint32_t)i;
+    } else {
+        k = (uint32_t)g.pkey_max;  // dead bucket: sorted behind every live cell
+        const uint32_t slot = atomicAdd(&removed[0], 1u);
+        if (slot < removed_cap) removed[1 + slot] = idx[pos];
+    }
+    key[pos] = k;
+    cellx[pos] = ci;
 }
 #endif
 
@@ -338,6 +371,10 @@ struct sphmw_ctx {
     bool allocated[NSLOT] = {};
     bool stale[NSLOT] = {};  // contents not up to date: skip in reorder, rebuild on demand
     bool dv_zero = true;     // Dv is known to be all-zero (never written since accelerate!)
+    // the keys, columns and removed list of the current positions were written by the force pass's
+    // advance (whole-domain multi-step call): the next cell-list build skips k_keys.  Consumed by that
+    // build; cleared by everything else that changes x
+    bool keys_from_advance = false;
 
     uint32_t *idx = nullptr, *idx_alt = nullptr;  // reference particle index of each position
     uint32_t *pos_of_idx = nullptr;               // inverse map (whole-domain contexts only), valid iff pos_valid
@@ -388,6 +425,17 @@ struct sphmw_ctx {
     int64_t pl_builds = 0;
     unsigned long long pl_overflow_seen = 0;  // overflow counter at the last look (queue rows adapt, cell_list.cu)
     int pl_format = 0;             // what the valid list holds: 0 global positions, 1 tile slots
+    // fluid work list of one cell-list generation (cell_list.cu, pair_list.cuh k_binary_list_fluid):
+    // the positions with type == fluid ascending, then the others ascending.  Built by every cell-list
+    // build once a fused WCSPH step has asked for it
+    bool want_fluid_list = false;
+    uint8_t *fluid_flag = nullptr;    // cap (+8): written by the gather
+    uint32_t *fluid_work = nullptr;   // cap
+    uint32_t *fluid_tiles = nullptr;  // fluid count per tile -> exclusive scan; fluid_tiles[tiles] = all
+    int64_t fluid_tiles_cap = 0;
+    const uint32_t *fluid_count = nullptr;  // device: the number of fluid positions
+    uint64_t fluid_gen = ~0ull;       // cell-list generation the list was built for
+    double fluid_value = 0.0;         // ... and the type value (Params::fluid) it was built with
     // neighbourhood tiles (tile_map.cuh): one record per block of TM_BLOCK particles
     uint32_t *tile_tab = nullptr;
     uint64_t tile_gen = ~0ull;     // cell-list generation the records were built for

@@ -90,6 +90,13 @@ struct PairOpBase {
     // packed neighbour records (pair_list.cuh): 0 the operator does not use them, 1 it needs
     // record A, 2 it needs A, B, C
     static constexpr int REC_KIND = 0;
+    // true only where finish() provably discards the pair sums of a particle whose type is not
+    // fluid: the replaying pass then skips the pair loop of such particles (pair_list.cuh
+    // k_binary_list_fluid) and runs init() + finish() alone, which leaves the same bits behind
+    static constexpr bool PAIRS_FOR_FLUID_ONLY = false;
+    // run by the list and walk kernels right after finish(), with the grid at hand
+    template <int DIM>
+    __device__ void after(const Grid &, const Fields &, const Params &, int64_t) const {}
     // shared-memory tiles (pair_tile.cuh): number of field arrays the operator stages (0: the
     // operator has no tiled variant)
     template <int DIM>
@@ -190,6 +197,8 @@ struct B_wcsph_density_fused : PairOpBase {
 // goes to the `out` field set because other threads still read the old one.
 struct B_wcsph_momentum_fused : PairOpBase {
     static constexpr int REC_KIND = 2;
+    // wcsph_force_finish keeps the old velocity of every non-fluid particle
+    static constexpr bool PAIRS_FOR_FLUID_ONLY = true;
     template <int DIM>
     __host__ __device__ static constexpr int tile_fields() { return DIM == 2 ? 9 : 9; }
     template <int DIM>
@@ -280,6 +289,14 @@ struct B_force_advance : Base {
             if (i < c.esc_lo || i >= c.esc_hi) atomicAdd(c.esc_counter, 1u);
         }
     }
+    // whole-domain call: the next cell list's key of the new position (k_keys of the next build, which
+    // then skips that launch; cell_list.cu)
+    template <int DIM>
+    __device__ void after(const Grid &g, const Fields &out, const Params &c, int64_t p) const {
+        if (c.key_out)
+            cell_key_whole<DIM>(g, out.s[S_X0][p], out.s[S_X1][p], DIM == 3 ? out.s[S_X2][p] : 0.0, p, c.key_out,
+                                c.cellx_out, c.key_removed, c.key_removed_cap, c.key_idx);
+    }
 };
 
 // ---- fast-arithmetic variants of the two fused passes (SPHMW_FLAG_FAST_MATH) ----------
@@ -337,6 +354,7 @@ struct B_wcsph_density_fast : PairOpBase {
 
 struct B_wcsph_momentum_fast : PairOpBase {
     static constexpr int REC_KIND = 2;
+    static constexpr bool PAIRS_FOR_FLUID_ONLY = true;  // as B_wcsph_momentum_fused
     template <int DIM>
     __host__ __device__ static constexpr int tile_fields() { return DIM == 2 ? 9 : 9; }
     template <int DIM>
