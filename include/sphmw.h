@@ -247,6 +247,29 @@ int sphmw_swap_removal_moves(int64_t n, const int64_t *removed, int64_t k, int64
  * "count" | "sum:<field>" | "max:<field>" */
 int sphmw_reduce(sphmw_ctx *ctx, const char *what, double *out);
 
+/* ≙ the point sum of src/core.jl:240-291: out[o*n + i] = sum over the particles within sys.h of
+ * point i (points[c*n + i], c = 0..2) of op o's term, in the reference's traversal order.
+ * The walk is _apply_binary! (core.jl:94-112) with the point in place of p: home cell find_key(x),
+ * the key_diff cells with only 1 <= key + dkey <= key_max checked, each cell in stored order,
+ * accepted when r <= sys.h, and no self-exclusion (a particle at r = 0 counts).  Each sum starts at
+ * 0.0; W = wendland2 (2D) | wendland3 (3D) of (sys.h, r); terms are folded left to right:
+ *   "count" 1.0 | "mW" m*W | "mW*<f>" (m*f)*W | "VW" (m/rho)*W | "VW*<f>" ((m/rho)*f)*W
+ * <f> is a scalar field name of sphmw_upload (ASCII or Julia spelling) or a vector component
+ * "v[c]", "Dv[c]", ... (c 0-based; c = 2 on a 2D context is SPHMW_E_INVALID).  Stale fields are
+ * brought up to date first, as for sphmw_reduce; fields never written read as zeros.
+ * A point outside the closed bounding box (a NaN coordinate, or in 2D a third coordinate != 0) gets
+ * NaN in every output — unlike the reference, where its key takes part in the linear key wrap.  A
+ * point without an accepted particle gets 0.0.
+ * points and out are host or device pointers (UVA decides).  With a host `out` the call blocks; with
+ * a device `out` it enqueues on the context's stream (a pinned host `points` buffer is copied before
+ * the call returns).  nops outside 1..SPHMW_POINT_OPS_MAX is SPHMW_E_INVALID, an unknown op
+ * SPHMW_E_UNSUPPORTED_OP, an unknown field SPHMW_E_UNKNOWN_FIELD; it needs a valid cell list
+ * (SPHMW_E_STATE after a move or an upload of x until sphmw_create_cell_list) and a whole-domain
+ * context (SPHMW_E_STATE on x-slabs).  n = 0 is a no-op.  The call changes no particle state. */
+#define SPHMW_POINT_OPS_MAX 8
+int sphmw_point_sum(sphmw_ctx *ctx, const char *const *ops, int32_t nops, const double *points, int64_t n,
+                    double *out);
+
 /* ≙ the exported smoothing kernels, evaluated on the device — src/kernels.jl.
  * name: wendland1|2|3, Dwendland1|2|3, rDwendland1|2|3, DDwendland3,
  * spline23|24, Dspline23|24, rDspline23|24.  h, r, out: n doubles (host). */

@@ -100,6 +100,7 @@ _SIGS = {
     "sphmw_comm_info": (C.c_int, [_P, C.POINTER(C.c_int64)]),
     "sphmw_comm_open_box": (C.c_int, [_P, C.c_int32]),
     "sphmw_reduce": (C.c_int, [_P, C.c_char_p, C.POINTER(C.c_double)]),
+    "sphmw_point_sum": (C.c_int, [_P, C.POINTER(C.c_char_p), C.c_int32, C.c_void_p, C.c_int64, C.c_void_p]),
     "sphmw_kernel_eval": (C.c_int, [C.c_char_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32]),
     "sphmw_pvd_open": (C.c_int, [_P, C.c_char_p]),
     "sphmw_pvd_save_frame": (C.c_int, [_P, C.POINTER(C.c_char_p), C.c_int32]),

@@ -22,7 +22,7 @@ ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 # an FMA; bit-exact neighbour sets and reproducible FP64 sums depend on it.
 NVCC_FLAGS = ARCH + ["-O3", "-std=c++17", "-lineinfo", "-fmad=false", "-Xcompiler", "-fPIC,-O2",
                      "-Xcudafe", "--diag_suppress=177", f"-I{ROOT / 'include'}", f"-I{CSRC}"]
-SOURCES = ["api.cu", "cell_list.cu", "pair_ops.cu", "halo.cu", "slab_comm.cu", "frame_async.cu", "lattice.cu", "frame_io.cpp", "grid_setup.cpp"]
+SOURCES = ["api.cu", "cell_list.cu", "pair_ops.cu", "halo.cu", "slab_comm.cu", "frame_async.cu", "lattice.cu", "point_sum.cu", "frame_io.cpp", "grid_setup.cpp"]
 
 
 def _nvcc() -> str:

@@ -334,6 +334,7 @@ extern "C" int sphmw_destroy(sphmw_ctx *c) {
     cudaFree(c->cell_start); cudaFree(c->scan_tmp); cudaFree(c->removed);
     cudaFree(c->mv_old); cudaFree(c->mv_new);
     cudaFree(c->d_counters); cudaFree(c->staging); cudaFree(c->reduce_tmp);
+    cudaFree(c->pt_pts); cudaFree(c->pt_out); cudaFree(c->pt_key); cudaFree(c->pt_order); cudaFree(c->pt_sort_tmp);
     cudaFree(c->fluid_flag); cudaFree(c->fluid_work); cudaFree(c->fluid_tiles);
     cudaFree(c->xq); cudaFree(c->pl.list); cudaFree(c->pl.list16); cudaFree(c->pl.cnt); cudaFree(c->tile_tab);
     for (int k = 0; k < 3; ++k) cudaFree(c->rec[k]);

@@ -163,25 +163,34 @@ __device__ __forceinline__ bool neighbour_pkey(const Grid &g, const CellCoord &c
     pk = pkey_ijk(g, i, j, k);
     return true;
 }
-// find_key + is_inside of one particle of a whole-domain context (structs.jl:97-106, geometry.jl:24-30):
-// the physical key and column of position pos, or — outside the box (closed intervals; NaN fails every
-// comparison) — the dead bucket, with its reference index appended to the removed list.  Shared by the
-// cell-list build (k_keys) and the force pass's advance, so both compute the same bits.
+// is_inside + find_key of a whole-domain context (geometry.jl:24-30, structs.jl:97-106): false outside the
+// box (closed intervals; NaN fails every comparison), else the cell (i, j, k) of the position.  Particles
+// (cell_key_whole) and sample points (point_sum.cuh) both call it, so a point and a particle at the same
+// coordinates get the same home cell bit for bit.
+template <int DIM>
+__host__ __device__ __forceinline__ bool cell_ijk_whole(const Grid &g, double x, double y, double z, int &i, int &j,
+                                                        int &k) {
+    if (!(g.box[0] <= x && x <= g.box[3] && g.box[1] <= y && y <= g.box[4] && g.box[2] <= z && z <= g.box[5]))
+        return false;
+    // IEEE division, then floor (never a reciprocal multiply)
+    i = (int)((long long)floor(x / g.h) - g.phase[0]);
+    j = (int)((long long)floor(y / g.h) - g.phase[1]);
+    k = DIM == 3 ? (int)((long long)floor(z / g.h) - g.phase[2]) : 0;
+    return true;
+}
+// find_key + is_inside of one particle of a whole-domain context: the physical key and column of
+// position pos, or — outside the box — the dead bucket, with its reference index appended to the removed
+// list.  Shared by the cell-list build (k_keys) and the force pass's advance, so both compute the same bits.
 template <int DIM>
 __device__ __forceinline__ void cell_key_whole(const Grid &g, double x, double y, double z, int64_t pos,
                                                uint32_t *__restrict__ key, uint32_t *__restrict__ cellx,
                                                uint32_t *__restrict__ removed, uint32_t removed_cap,
                                                const uint32_t *__restrict__ idx) {
-    const bool inside = g.box[0] <= x && x <= g.box[3] && g.box[1] <= y && y <= g.box[4] && g.box[2] <= z &&
-                        z <= g.box[5];
+    int i, j, kk;
     uint32_t k, ci = 0;
-    if (inside) {
-        // IEEE division, then floor (never a reciprocal multiply)
-        const long long i = (long long)floor(x / g.h) - g.phase[0];
-        const long long j = (long long)floor(y / g.h) - g.phase[1];
-        const long long kk = DIM == 3 ? (long long)floor(z / g.h) - g.phase[2] : 0;
+    if (cell_ijk_whole<DIM>(g, x, y, z, i, j, kk)) {
         // structs.jl:102 gives the reference key i + Lx*(j + Ly*k); stored is its physical image
-        k = pkey_ijk(g, (int)i, (int)j, (int)kk);
+        k = pkey_ijk(g, i, j, kk);
         ci = (uint32_t)i;
     } else {
         k = (uint32_t)g.pkey_max;  // dead bucket: sorted behind every live cell
@@ -442,6 +451,12 @@ struct sphmw_ctx {
 
     double *staging = nullptr;  // 3*cap doubles
     double *reduce_tmp = nullptr;
+    // point sums (point_sum.cu): grow-only scratch for host points and outputs, keys and order
+    double *pt_pts = nullptr, *pt_out = nullptr;
+    uint32_t *pt_key = nullptr, *pt_order = nullptr;  // 2 x pt_cap each: as computed, sorted
+    void *pt_sort_tmp = nullptr;
+    int64_t pt_cap = 0, pt_out_cap = 0;
+    size_t pt_sort_tmp_bytes = 0;
 
     bool cell_list_valid = false;
     bool count_pairs = false;

@@ -333,6 +333,38 @@ function add_new_particles!(sys::ParticleSystem)
     return n[]
 end
 
+"""
+    point_sums(sys, ops::Vector{String}, X::AbstractMatrix) -> Matrix{Float64}
+
+≙ `sum(sys, f, x)` (core.jl:240-291) at every column of the 3 x n matrix `X`, on the device
+(sphmw_point_sum): row o of the result is op o summed over the particles within sys.h of each point, in
+the reference's traversal order, with no self-exclusion.  Ops: "count", "mW", "VW", "mW*<f>",
+"VW*<f>" (term m W, (m f) W, (m/ρ) W, ((m/ρ) f) W; W = wendland2 in 2D, wendland3 in 3D); <f> is a
+field name ("ρ′", "θ", ...) or a vector component "v[0]" (0-based).  Points outside the domain's
+bounding box give NaN.  Needs a current cell list (create_cell_list! after the last move!).
+"""
+function point_sums(sys::ParticleSystem, ops::Vector{String}, X::AbstractMatrix)
+    size(X, 1) == 3 || throw(SphmwError(-1, "point_sums: X must be 3 x n"))
+    before_device_call!(sys)
+    n = size(X, 2)
+    soa = Vector{Float64}(undef, 3n)
+    for i in 1:n, c in 1:3
+        soa[(c - 1) * n + i] = X[c, i]
+    end
+    out = Vector{Float64}(undef, length(ops) * n)
+    GC.@preserve ops begin
+        ptrs = [Base.unsafe_convert(Cstring, Base.cconvert(Cstring, o)) for o in ops]
+        check(ccall((:sphmw_point_sum, libsphmw), Cint, (Ptr{Cvoid}, Ptr{Cstring}, Int32, Ptr{Float64}, Int64, Ptr{Float64}),
+                    sys.ctx, ptrs, length(ptrs), soa, n, out))
+    end
+    return permutedims(reshape(out, n, length(ops)))
+end
+"≙ `sum(sys, f, x)` of core.jl:240-291 for a device op string (see point_sums)"
+Base.sum(sys::ParticleSystem, op::String, x::RealVector)::Float64 =
+    point_sums(sys, [op], reshape([x[1], x[2], x[3]], 3, 1))[1, 1]
+Base.sum(sys::ParticleSystem, f::Function, x) =
+    throw(SphmwError(-3, "sum: the closure $(nameof(f)) cannot run on the device; a point sum takes a device op string (\"mW\", \"VW*<field>\", ...: see point_sums)"))
+
 assemble_matrix(args...) = throw(SphmwError(-3, "assemble_matrix (ISPH, core.jl:175-246) is outside the device path"))
 assemble_vector(args...) = throw(SphmwError(-3, "assemble_vector (ISPH, core.jl:248-291) is outside the device path"))
 

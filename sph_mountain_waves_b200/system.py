@@ -312,6 +312,46 @@ class ParticleSystem:
         check(_capi.lib().sphmw_reduce(self.ctx, what.encode(), C.byref(out)))
         return out.value
 
+    def point_sum(self, points, ops):
+        """≙ sum(sys, f, x) of src/core.jl:240-291 at many points (sphmw_point_sum): row o of the result
+        is op o ("count", "mW", "VW", "mW*<field>", "VW*<field>", e.g. "VW*v[1]") summed over the particles
+        within h of each point, in the reference's traversal order.  `points` is an (n, 3) float64 numpy
+        array, or a CUDA torch tensor, which stays on the device (the result is then a CUDA tensor).
+        Points outside the box give NaN.  Needs a current cell list."""
+        self._flush()
+        ops = [ops] if isinstance(ops, str) else list(ops)
+        arr = (C.c_char_p * len(ops))(*[o.encode() for o in ops])
+        if type(points).__module__.split(".")[0] == "torch":
+            import torch
+            if not points.is_cuda or points.dtype != torch.float64 or points.dim() != 2 or points.shape[1] != 3:
+                raise ValueError("points: expected a CUDA float64 tensor of shape (n, 3)")
+            soa = points.t().contiguous()
+            out = torch.empty((len(ops), points.shape[0]), dtype=torch.float64, device=points.device)
+            torch.cuda.current_stream(points.device).synchronize()  # the library runs on its own stream
+            check(_capi.lib().sphmw_point_sum(self.ctx, arr, len(ops), C.c_void_p(soa.data_ptr()),
+                                              points.shape[0], C.c_void_p(out.data_ptr())))
+            self.sync()
+            return out
+        pts = np.asarray(points, dtype=np.float64)
+        if pts.ndim != 2 or pts.shape[1] != 3:
+            raise ValueError(f"points: expected shape (n, 3), got {pts.shape}")
+        soa = np.ascontiguousarray(pts.T)
+        out = np.empty((len(ops), pts.shape[0]), dtype=np.float64)
+        check(_capi.lib().sphmw_point_sum(self.ctx, arr, len(ops), _capi.ptr(soa), pts.shape[0], _capi.ptr(out)))
+        return out
+
+    def interpolate(self, points, fields) -> dict:
+        """Shepard interpolant Σ VW*f / Σ VW of each field at the points, from one point_sum call
+        (len(fields) + 1 <= 8 ops); NaN where no particle is within h or the point is outside the box."""
+        fields = [fields] if isinstance(fields, str) else list(fields)
+        s = self.point_sum(points, ["VW"] + [f"VW*{f}" for f in fields])
+        den = s[0]
+        if isinstance(s, np.ndarray):
+            with np.errstate(invalid="ignore", divide="ignore"):
+                return {f: np.where(den == 0.0, np.nan, s[k + 1] / den) for k, f in enumerate(fields)}
+        nan = den.new_full((), float("nan"))
+        return {f: (s[k + 1] / den).where(den != 0.0, nan) for k, f in enumerate(fields)}
+
     def key_tables(self):
         ph = (C.c_int64 * 3)()
         lim = (C.c_int64 * 3)()
