@@ -244,7 +244,11 @@ int sphmw_swap_removal_moves(int64_t n, const int64_t *removed, int64_t k, int64
 
 /* ≙ avg_velocity / max_velocity / length(sys.particles)
  * (wcsph_perturbed_witch.jl:338-350,377).  what: "avg_speed" | "max_speed" |
- * "count" | "sum:<field>" | "max:<field>" */
+ * "count" | "sum:<field>" | "max:<field>" (<field> a scalar field, else SPHMW_E_UNKNOWN_FIELD).
+ * Sums are FP64 in a fixed tree; max propagates NaN and orders -0.0 below +0.0, as Julia's max.
+ * Stale fields are brought up to date first; a field never written reads as 0.0.  x-slab
+ * contexts are refused with SPHMW_E_STATE: their particles include ghost copies (the owned count
+ * is sphmw_slab_counts). */
 int sphmw_reduce(sphmw_ctx *ctx, const char *what, double *out);
 
 /* ≙ the point sum of src/core.jl:240-291: out[o*n + i] = sum over the particles within sys.h of

@@ -570,9 +570,12 @@ extern "C" int sphmw_download(sphmw_ctx *c, const char *field, double *buf, int6
 // reductions — avg_velocity/max_velocity (wcsph_perturbed_witch.jl:338-350)
 // ---------------------------------------------------------------------------
 // mode 0: sum of a, 1: max of a, 2: sum |v|, 3: max |v|
-// Julia's max propagates NaN (wcsph_perturbed_witch.jl:345-350 uses it for max_velocity); fmax drops it
+// Julia's max propagates NaN (wcsph_perturbed_witch.jl:345-350 uses it for max_velocity); fmax drops it.
+// Like Julia's max it also orders -0.0 below +0.0, so that the result does not depend on where the
+// zeros sit in the reduction tree.
 __device__ __forceinline__ double nanmax(double a, double b) {
     if (a != a || b != b) return a + b;
+    if (a == b) return signbit(a) ? b : a;
     return a < b ? b : a;
 }
 __global__ void k_reduce(const double *a, const double *b, const double *cc, int64_t n, int mode,
@@ -629,6 +632,12 @@ static int reduce_run(sphmw_ctx *c, const double *a, const double *b, const doub
 
 extern "C" int sphmw_reduce(sphmw_ctx *c, const char *what, double *out) {
     if (!c || !what || !out) { sphmw_set_error("null argument"); return SPHMW_E_INVALID; }
+    if (c->slab_lo >= 0) {
+        // k_reduce runs over the resident particles, ghost columns included
+        sphmw_set_error("reduce: x-slab contexts are not supported (the resident particles include ghost copies); "
+                        "use sphmw_slab_counts for the owned count, or reduce on a whole-domain context");
+        return SPHMW_E_STATE;
+    }
     CUDA_TRY(cudaSetDevice(c->device));
     if (!strcmp(what, "count")) {
         *out = (double)c->n;

@@ -302,11 +302,12 @@ struct B_force_advance : Base {
 // ---- fast-arithmetic variants of the two fused passes (SPHMW_FLAG_FAST_MATH) ----------
 // Same neighbour set (the cut-off test stays exact) and the same summation ORDER, but the
 // closure bodies use fused multiply-adds, reciprocals instead of divisions and one rsqrt,
-// like the reference's own @fastmath kernels (kernels.jl:108-195).  Every operation is
-// accurate to ~1 ulp, so rho and v stay within a few 1e-16 relative of the strict path per
-// pair — far inside the north star's 1e-10 per step — while the FP64 instruction count of
-// the accepted-pair path drops ~2.5x.  Results remain deterministic and independent of the
-// number of ranks (the code path is the same everywhere).
+// like the reference's own @fastmath kernels (kernels.jl:108-195).  Per particle, rho, h, P and
+// v stay as close to an extended-precision evaluation as the strict path's: the median error is
+// below 1.0 (rho) and 0.6 (v) units of 2^-53 times the sum of the pair terms' magnitudes
+// (tests/test_xp_wcsph_emulated.py, tests/test_gpu_xp_wcsph.py; DESIGN.md §2) — while the FP64
+// instruction count of the accepted-pair path drops ~2.5x.  Results remain deterministic and
+// independent of the number of ranks (the code path is the same everywhere).
 __device__ __forceinline__ double fast_sqrt_pos(double a) {
     // a > 0 finite in the accepted-pair path (a == 0 only for coincident particles)
     if (a <= 0.0) return a == 0.0 ? 0.0 : sqrt(a);
